@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the driver's benchmark contract for the render hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 One "step" = one full render of the workload (generate .. extend/shadow .. shade
 .. accumulate .. tonemap) on synthetic input: the reference's default scene
@@ -13,6 +13,13 @@ replicated, per-GPU accumulation buffers summed inside the timed step with one
 NCCL all-reduce issued by the LIBRARY (rtb_comm_allreduce_f32, include/rtb.h),
 then tonemapped.  torch.distributed only carries the barrier, the NCCL id and
 the timing exchange.
+
+--dump-outputs DIR (rank 0) writes what the last timed step computed as DIR/<name>.npy, float32: image.npy (the
+tonemapped frame) and accum.npy (the summed radiance it was tonemapped from), H x W x 3 each.  When the two exceed
+64 MB (64,000,000 bytes) together, both hold the same fixed, seeded sample of pixels as rows, and pixel_index.npy
+(float64) says which; a full-frame dump removes a pixel_index.npy an earlier dump left in DIR.
+The scene, camera and sample seeds are fixed, so two builds run with the same arguments can be compared output for
+output.
 
 Prints ONE JSON line (rank 0).
   value      Mrays/s (extend + shadow rays actually traversed by all ranks) / device time
@@ -484,6 +491,30 @@ class Job:
         self.scene.close()
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs: the most it writes in all
+
+
+def dump_outputs(outdir, job):
+    """the last step's tonemapped image and accumulation buffer (see --dump-outputs in the module docstring)"""
+    os.makedirs(outdir, exist_ok=True)
+    npix = job.W * job.H
+    out = {"image": job.out, "accum": job.accum}
+    out = {k: v.view(npix, 3).cpu().numpy() for k, v in out.items()}
+    per_pixel = sum(a.itemsize * 3 for a in out.values())
+    if npix * per_pixel > DUMP_BYTES:
+        keep = (DUMP_BYTES - 4096) // (per_pixel + 8)  # (4096: room for the .npy headers)
+        idx = np.sort(np.random.default_rng(0).choice(npix, keep, replace=False))
+        out = {k: a[idx] for k, a in out.items()}
+        out["pixel_index"] = idx.astype(np.float64)
+    else:
+        out = {k: a.reshape(job.H, job.W, 3) for k, a in out.items()}
+        stale = os.path.join(outdir, "pixel_index.npy")
+        if os.path.exists(stale):
+            os.remove(stale)
+    for k, a in out.items():
+        np.save(os.path.join(outdir, k + ".npy"), a)
+
+
 def e2e_leg(rig, job, steps):
     """end to end through the public API from pinned host buffers, every step: upload + BVH build + render + D2H.
     N = 1: rtb_scene_create + rtb_render.  N > 1, one process per GPU as the driver launches them: every rank
@@ -580,7 +611,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `secondary` (C3) and `strong` records of the default workload")
     ap.add_argument("--flags", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's image and accumulation buffer to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("bench.py: --dump-outputs writes what --impl ours computes")
     # W >= 3 (timing contract); the multi-second C5 steps may run with fewer to fit a GPU lease
     args.warmup = max(args.warmup, 3) if args.impl == "ours" and args.workload not in STRONG else args.warmup
     if args.impl == "reference":
@@ -599,6 +635,8 @@ def main():
     job = Job(rig, args.workload, spp, total_spp, rank * spp, pool=args.pool, flags=args.flags)
     res = job.timed(args.steps, args.warmup, sampler=ClockSampler(rig.local_rank) if rank == 0 else None, spin=True)
     stats = res["stats"]
+    if args.dump_outputs and rank == 0:  # before the legs below reuse the job's buffers
+        dump_outputs(args.dump_outputs, job)
     launches = int(sum(s.kernel_launches for s in stats) + 2 * args.steps)  # + fold into the caller's buffer + tonemap per step
     e2e = e2e_leg(rig, job, args.steps)
     one_proc = one_process_leg(rig, job, args.steps)

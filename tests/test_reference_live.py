@@ -29,7 +29,7 @@ def run_harness(scene_file, *cmd):
 @pytest.fixture(scope="module")
 def setup(gpu, bunny, tmp_path_factory):
     if not os.path.exists(harness_path()):
-        pytest.skip("oracle/_ref/ref_harness not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/ref_harness not built (needs the original rtcuda sources at build time, oracle/Makefile REF)")
     td = tmp_path_factory.mktemp("ref")
     hs = gpu.host_scene(capi.RTB_SCENE_S1, *bunny)
     sf = str(td / "s1.rtbs")
