@@ -128,7 +128,13 @@ typedef struct rtb_instanced_scene_desc {
 } rtb_instanced_scene_desc;
 
 /* BVH builder selection (rtb_build_params.builder) */
-enum { RTB_BUILDER_PLOC = 0 }; /* the only builder so far; other values are rejected */
+enum {
+    RTB_BUILDER_PLOC = 0,       /* parallel locally-ordered clustering over Morton order (default) */
+    RTB_BUILDER_BINNED_SAH = 1  /* top-down binned SAH (32 bins per axis, split down to single primitives): a tree
+                                   for faster traces at a longer build time; ploc_radius is ignored, ploc_iterations
+                                   is 0.  Exact-t ties at shared edges can resolve differently from the reference, as
+                                   with RTB_COLLAPSE_SAH_OPTIMAL (DESIGN.md 4.1) */
+};
 
 /* how the binary tree is collapsed into 8-wide nodes (rtb_build_params.collapse) */
 enum {

@@ -20,6 +20,8 @@ RTB_MATTE, RTB_MIRROR, RTB_GLASS, RTB_GLOSSY = 0, 1, 2, 3
 RTB_RENDER_PIXEL_CENTRE, RTB_RENDER_NO_SHADOW, RTB_RENDER_NONPERSISTENT, RTB_RENDER_COUNT_WORK = 1, 2, 4, 8
 RTB_RENDER_SINGLE_PIPELINE = 16
 RTB_RENDER_TRUE_MIS, RTB_RENDER_RR_TERMINATE, RTB_RENDER_DETERMINISTIC = 32, 64, 128
+RTB_BUILDER_PLOC, RTB_BUILDER_BINNED_SAH = 0, 1
+RTB_COLLAPSE_LARGEST_FIRST, RTB_COLLAPSE_SAH_OPTIMAL = 0, 1
 
 
 class Material(C.Structure):

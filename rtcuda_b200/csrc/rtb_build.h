@@ -8,6 +8,9 @@
 //   3. PLOC           parallel locally-ordered clustering (Meister & Bittner
 //                     2018): nearest neighbour within a window of the Morton
 //                     order, merge mutual pairs, compact; repeat to one root
+//   3'. binned SAH    (RTB_BUILDER_BINNED_SAH, instead of 2-3) top-down
+//                     32-bin SAH splits down to single primitives: large
+//                     ranges level by level, small ones one block each
 //   4. collapse plan  (optional, RTB_COLLAPSE_SAH_OPTIMAL; default is the greedy
 //                     "largest child first" of step 5)
 //                     bottom-up dynamic programme over the binary tree (after
@@ -231,6 +234,211 @@ RTB_HD void ploc_merge_body(const PlocArgs &a, int n_leaves, int i) {
     (void)n_leaves;
 }
 
+// ------------------------------------------------------------ 3'. binned SAH (RTB_BUILDER_BINNED_SAH)
+// Top-down, instead of steps 2-3: a node's primitives are a contiguous range [begin, end) of a primitive index array; its
+// split is the cheapest of 31 planes per axis (cost A_L N_L + A_R N_R) between 32 bins over its centroid extent, and
+// depends on nothing but its primitive set and centroid bounds (counts and boxes are accumulated as integers / ordered
+// ints, so the order of accumulation is free).  A stable partition of the range then gives the two children.  Ranges go
+// down to single primitives: a range of one primitive at position p is leaf node p (left = idx[p]); inner nodes take ids
+// n .. 2n-2.  Large ranges are split level by level by the whole device, small ones (<= kSahSmall) by one block each.
+constexpr int kSahBins = 32;
+constexpr int kSahBinWords = 7;                              // count, box lo xyz, box hi xyz (ordered ints)
+constexpr int kSahBinsWords = 3 * kSahBins * kSahBinWords;   // a node's bins, [axis][bin][word]
+constexpr int kSahSmall = 1024;                              // ranges up to this size are finished in one block
+constexpr int kSahChunk = 4096;                              // primitives per block of a level's kernels
+// Binary depth beyond which the 8-wide tree cannot fit the traversal stack: the collapse turns at most 7 binary levels
+// into one 8-wide level, and kStackSize 8-wide levels are already too deep.
+constexpr int kSahMaxDepth = 7 * kStackSize;
+struct SahRange { int32_t begin, end, id, depth; };
+struct SahTask {          // a large range of one level
+    SahRange r;
+    int32_t bnd[12];      // ordered ints: box lo xyz, box hi xyz, centroid lo xyz, centroid hi xyz
+    int32_t blk0;         // its first block in the level's block -> task map
+    int32_t axis, plane, nl;  // the split: axis -1 = by position; nl = primitives going left
+};
+struct SahArgs {
+    const F4 *prim_lo, *prim_hi;
+    int32_t *idx, *idx2;          // [n] primitive at each position; scatter target
+    int32_t *flags, *scan;        // [n] "goes left" and its exclusive scan (large ranges)
+    B2Node *nodes; int32_t *count;
+    int32_t *depth;               // [n-1] depth of inner node id, at [id - n]
+    int32_t *node_counter;
+    const SahTask *tin_c; SahTask *tin, *tout;  // this level's tasks (tin_c == tin), the next level's
+    const int32_t *blk_in; int32_t *blk_out;    // block -> task
+    const int32_t *n_tin, *n_blk_in;            // counts of this level (device memory)
+    int32_t *n_tout, *n_blk_out;                // next level's counts
+    int32_t *n_clear, *n_blk_clear;             // the counts of the level after the next, cleared by this level
+    int32_t *bins;                // [task][kSahBinsWords], neutral between uses
+    SahRange *small; int32_t *n_small;
+    int32_t n;
+};
+RTB_HD V3 sah_centroid(const F4 &lo, const F4 &hi) {  // as morton_body
+    return v3(fmul(0.5f, fadd(lo.x, hi.x)), fmul(0.5f, fadd(lo.y, hi.y)), fmul(0.5f, fadd(lo.z, hi.z)));
+}
+RTB_HD float v3_at(const V3 &v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : v.z); }
+// bins per unit of centroid extent on axis k, 0 when the axis is unusable (no extent, or a scale that is not finite)
+RTB_HD float sah_scale(const int32_t *bnd, int k) {
+    const float e = fsub(ordered_to_float(bnd[9 + k]), ordered_to_float(bnd[6 + k]));
+    const float s = e > 0.f ? fdiv((float)kSahBins, e) : 0.f;
+    return s <= FLT_MAX ? s : 0.f;
+}
+RTB_HD int sah_bin(float c, float cmin, float scale) {
+    const int b = (int)fmul(fsub(c, cmin), scale);
+    return b < 0 ? 0 : (b >= kSahBins ? kSahBins - 1 : b);
+}
+RTB_HD void sah_bnd_init(int32_t *b) {
+    for (int k = 0; k < 3; ++k) { b[k] = b[6 + k] = float_to_ordered(FLT_MAX); b[3 + k] = b[9 + k] = float_to_ordered(-FLT_MAX); }
+}
+RTB_HD void sah_bin_init(int32_t *w) {
+    w[0] = 0;
+    for (int k = 0; k < 3; ++k) { w[1 + k] = float_to_ordered(FLT_MAX); w[4 + k] = float_to_ordered(-FLT_MAX); }
+}
+// one primitive into the bins of the usable axes (atomics: shared memory on the device)
+RTB_HD void sah_bin_add(int32_t *bins, const F4 &lo, const F4 &hi, const int32_t *bnd, const float *scale) {
+    const V3 c = sah_centroid(lo, hi);
+    const int32_t l[3] = {float_to_ordered(lo.x), float_to_ordered(lo.y), float_to_ordered(lo.z)};
+    const int32_t h[3] = {float_to_ordered(hi.x), float_to_ordered(hi.y), float_to_ordered(hi.z)};
+    for (int a = 0; a < 3; ++a) {
+        if (scale[a] <= 0.f) continue;
+        int32_t *w = bins + (a * kSahBins + sah_bin(v3_at(c, a), ordered_to_float(bnd[6 + a]), scale[a])) * kSahBinWords;
+        atomic_add_i(w, 1);
+        for (int k = 0; k < 3; ++k) { atomic_min_i(w + 1 + k, l[k]); atomic_max_i(w + 4 + k, h[k]); }
+    }
+}
+RTB_HD void sah_bin_merge(int32_t *acc, const int32_t *w) {
+    acc[0] += w[0];
+    for (int k = 0; k < 3; ++k) { acc[1 + k] = acc[1 + k] < w[1 + k] ? acc[1 + k] : w[1 + k]; acc[4 + k] = acc[4 + k] > w[4 + k] ? acc[4 + k] : w[4 + k]; }
+}
+RTB_HD float sah_inf() { return i2f(0x7f800000); }
+// cost of a plane with the bins l (left of it) and r (right of it) merged; +inf when a side is empty or the cost overflows
+RTB_HD float sah_plane_cost(const int32_t *l, const int32_t *r) {
+    if (l[0] <= 0 || r[0] <= 0) return sah_inf();
+    const float al = half_area(fsub(ordered_to_float(l[4]), ordered_to_float(l[1])), fsub(ordered_to_float(l[5]), ordered_to_float(l[2])),
+                               fsub(ordered_to_float(l[6]), ordered_to_float(l[3])));
+    const float ar = half_area(fsub(ordered_to_float(r[4]), ordered_to_float(r[1])), fsub(ordered_to_float(r[5]), ordered_to_float(r[2])),
+                               fsub(ordered_to_float(r[6]), ordered_to_float(r[3])));
+    const float c = ffma(al, (float)l[0], fmul(ar, (float)r[0]));
+    return c <= FLT_MAX ? c : sah_inf();
+}
+struct SahSplit { int32_t axis, plane, nl; };
+// the split of a range of `size` primitives from its bins: lowest cost, ties to the lowest axis, then the lowest plane;
+// without a usable plane, the range is halved by position
+RTB_HD SahSplit sah_choose(const int32_t *bins, const float *scale, int size) {
+    SahSplit s; s.axis = -1; s.plane = 0; s.nl = size / 2;
+    float best = sah_inf();
+    for (int a = 0; a < 3; ++a) {
+        if (scale[a] <= 0.f) continue;
+        const int32_t *b = bins + a * kSahBins * kSahBinWords;
+        int32_t right[kSahBins][kSahBinWords];  // right[k]: bins k .. 31
+        sah_bin_init(right[kSahBins - 1]);
+        sah_bin_merge(right[kSahBins - 1], b + (kSahBins - 1) * kSahBinWords);
+        for (int k = kSahBins - 2; k >= 0; --k) {
+            for (int w = 0; w < kSahBinWords; ++w) right[k][w] = right[k + 1][w];
+            sah_bin_merge(right[k], b + k * kSahBinWords);
+        }
+        int32_t left[kSahBinWords];
+        sah_bin_init(left);
+        for (int k = 0; k + 1 < kSahBins; ++k) {
+            sah_bin_merge(left, b + k * kSahBinWords);
+            const float c = sah_plane_cost(left, right[k + 1]);
+            if (c < best) { best = c; s.axis = a; s.plane = k; s.nl = left[0]; }
+        }
+    }
+    return s;
+}
+// does the primitive at offset `off` of its range (box lo / hi) go to the left child?
+RTB_HD bool sah_goes_left(const SahSplit &s, int off, const F4 &lo, const F4 &hi, const int32_t *bnd) {
+    if (s.axis < 0) return off < s.nl;
+    const float c = v3_at(sah_centroid(lo, hi), s.axis);
+    return sah_bin(c, ordered_to_float(bnd[6 + s.axis]), sah_scale(bnd, s.axis)) <= s.plane;
+}
+// box and centroid bounds of one primitive into b (plain min / max: the caller reduces)
+RTB_HD void sah_bnd_add(int32_t *b, const F4 &lo, const F4 &hi) {
+    const V3 c = sah_centroid(lo, hi);
+    const int32_t v[12] = {float_to_ordered(lo.x), float_to_ordered(lo.y), float_to_ordered(lo.z), float_to_ordered(hi.x),
+                           float_to_ordered(hi.y), float_to_ordered(hi.z), float_to_ordered(c.x), float_to_ordered(c.y),
+                           float_to_ordered(c.z), float_to_ordered(c.x), float_to_ordered(c.y), float_to_ordered(c.z)};
+    for (int k = 0; k < 3; ++k) {
+        b[k] = b[k] < v[k] ? b[k] : v[k]; b[6 + k] = b[6 + k] < v[6 + k] ? b[6 + k] : v[6 + k];
+        b[3 + k] = b[3 + k] > v[3 + k] ? b[3 + k] : v[3 + k]; b[9 + k] = b[9 + k] > v[9 + k] ? b[9 + k] : v[9 + k];
+    }
+}
+// inner node r (box from bnd, split after nl primitives): writes the node, its count and depth, and its two children into
+// ch; a child of one primitive is the leaf at its position, a larger one takes an id from *ids
+RTB_HD void sah_make_node(const SahArgs &a, const SahRange &r, const int32_t *bnd, int nl, int32_t *ids, SahRange *ch) {
+    ch[0].begin = r.begin; ch[0].end = r.begin + nl;
+    ch[1].begin = r.begin + nl; ch[1].end = r.end;
+    for (int k = 0; k < 2; ++k) {
+        ch[k].depth = r.depth + 1;
+        ch[k].id = ch[k].end - ch[k].begin == 1 ? ch[k].begin : atomic_add_i(ids, 1);
+    }
+    B2Node m;
+    m.lox = ordered_to_float(bnd[0]); m.loy = ordered_to_float(bnd[1]); m.loz = ordered_to_float(bnd[2]); m.left = ch[0].id;
+    m.hix = ordered_to_float(bnd[3]); m.hiy = ordered_to_float(bnd[4]); m.hiz = ordered_to_float(bnd[5]); m.right = ch[1].id;
+    a.nodes[r.id] = m;
+    a.count[r.id] = r.end - r.begin;
+    a.depth[r.id - a.n] = r.depth;
+}
+// a child made by a level: to the next level (with its blocks), to the small ranges, or nothing (a leaf)
+RTB_HD void sah_push_child(const SahArgs &a, const SahRange &c) {
+    const int size = c.end - c.begin;
+    if (size <= 1) return;
+    if (size <= kSahSmall) { a.small[atomic_add_i(a.n_small, 1)] = c; return; }
+    const int t = atomic_add_i(a.n_tout, 1), nb = (size + kSahChunk - 1) / kSahChunk;
+    SahTask T;
+    T.r = c; sah_bnd_init(T.bnd);
+    T.blk0 = atomic_add_i(a.n_blk_out, nb);
+    T.axis = -1; T.plane = 0; T.nl = 0;
+    a.tout[t] = T;
+    for (int k = 0; k < nb; ++k) a.blk_out[T.blk0 + k] = t;
+}
+// first block of the build: root range, counters
+struct SahRootK {
+    SahArgs a; int32_t *root;
+    RTB_HD void operator()(int i) const {
+        if (i != 0) return;
+        *a.n_small = 0;
+        if (a.n == 1) { *root = 0; return; }
+        *root = a.n;
+        *a.node_counter = a.n + 1;
+        SahRange r; r.begin = 0; r.end = a.n; r.id = a.n; r.depth = 0;
+        sah_push_child(a, r);  // (the "next level" of the root's push is level 0)
+    }
+};
+struct SahIotaK { int32_t *p; int n; RTB_HD void operator()(int i) const { if (i < n) p[i] = i; } };
+struct SahBinsInitK { int32_t *bins; int n; RTB_HD void operator()(int i) const { if (i < n) sah_bin_init(bins + (size_t)i * kSahBinWords); } };
+// leaf node p = the primitive that ended at position p
+struct SahLeafK {
+    SahArgs a;
+    RTB_HD void operator()(int p) const {
+        if (p >= a.n) return;
+        const int g = a.idx[p];
+        const F4 lo = a.prim_lo[g], hi = a.prim_hi[g];
+        B2Node b;
+        b.lox = lo.x; b.loy = lo.y; b.loz = lo.z; b.left = g;
+        b.hix = hi.x; b.hiy = hi.y; b.hiz = hi.z; b.right = -1;
+        a.nodes[p] = b;
+        a.count[p] = 1;
+    }
+};
+// collapse plan order: inner nodes deepest first (sort key), and where each depth starts in that order
+struct SahDepthKeyK {
+    const int32_t *depth; uint64_t *keys; int32_t *vals; int n_inner, n;
+    RTB_HD void operator()(int i) const {
+        if (i >= n_inner) return;
+        const int d = depth[i] < kSahMaxDepth + 1 ? depth[i] : kSahMaxDepth + 1;
+        keys[i] = (uint64_t)(kSahMaxDepth + 1 - d);
+        vals[i] = n + i;
+    }
+};
+struct SahGroupK {
+    const uint64_t *keys; int32_t *first; int n_inner;
+    RTB_HD void operator()(int i) const {
+        if (i >= n_inner) return;
+        if (i == 0 || keys[i - 1] != keys[i]) first[keys[i]] = i;
+    }
+};
+
 // ------------------------------------------------------------ 4. collapse plan
 // cost[n][i-1], i = 1..7: SAH cost of subtree n laid out in at most i child
 // slots.  plan[n][i-1]: kPlanLeaf / kPlanInner (one slot), k = 1..6 (split:
@@ -244,6 +452,7 @@ struct PlanArgs {
     uint8_t *plan;    // [num binary nodes][8]
     int32_t first, n; // this launch covers binary nodes first .. first+n-1 (one PLOC round: children are older)
     int32_t max_leaf;
+    const int32_t *order;  // null: the nodes are ids first ..; else order[first ..] (the binned-SAH tree: one depth per launch)
 };
 RTB_HD void plan_child_costs(const PlanArgs &a, int c, float *d) {
     const B2Node x = a.nodes[c];
@@ -256,7 +465,7 @@ RTB_HD void plan_child_costs(const PlanArgs &a, int c, float *d) {
 }
 RTB_HD void plan_body(const PlanArgs &a, int tid) {
     if (tid >= a.n) return;
-    const int id = a.first + tid;
+    const int id = a.order ? a.order[a.first + tid] : a.first + tid;
     const B2Node self = a.nodes[id];
     if (self.right < 0) return;
     float dl[7], dr[7];

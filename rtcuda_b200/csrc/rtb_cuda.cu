@@ -30,6 +30,7 @@
 
 #include <cub/block/block_scan.cuh>
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 
 #include "rtb_engine.h"
@@ -617,6 +618,231 @@ __global__ void __launch_bounds__(kBlock) k_collapse_level(CollapseArgs a, int32
     for (int i = blockIdx.x * kBlock + threadIdx.x; i < n; i += gridDim.x * kBlock) collapse_body(a, i);
 }
 
+// ---- binned SAH builder (RTB_BUILDER_BINNED_SAH, rtb_build.h 3') ----
+// A level of large ranges: every range has ceil(size / kSahChunk) blocks (blk_in: block -> range).  k_sah_bounds reduces
+// box and centroid bounds per block (12 atomics per block and range), k_sah_bin bins in shared memory and flushes once
+// per block and range, k_sah_split chooses with one warp per range and makes the children, k_sah_flag / a scan /
+// k_sah_scatter / k_sah_copy partition every range stably in place.
+constexpr int kSahBlock = 256;
+__device__ __forceinline__ bool sah_block_range(const SahArgs &a, int &t, int &p0, int &p1) {
+    if ((int)blockIdx.x >= *a.n_blk_in) return false;
+    t = a.blk_in[blockIdx.x];
+    const SahRange r = a.tin_c[t].r;
+    p0 = r.begin + ((int)blockIdx.x - a.tin_c[t].blk0) * kSahChunk;
+    p1 = min(p0 + kSahChunk, r.end);
+    return true;
+}
+__device__ __forceinline__ void sah_load_bnd(const SahTask &T, int32_t *bnd, float *scale) {
+#pragma unroll
+    for (int k = 0; k < 12; ++k) bnd[k] = T.bnd[k];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) scale[k] = sah_scale(bnd, k);
+}
+// warp-wide sah_choose: lane k holds bin k of an axis; prefix / suffix merges by shuffles (integer sums and min / max:
+// exact in any order), the same costs and the same tie rule (lowest cost, then lowest axis, then lowest plane)
+__device__ __forceinline__ SahSplit sah_choose_warp(const int32_t *bins, const float *scale, int size, int lane) {
+    SahSplit s; s.axis = -1; s.plane = 0; s.nl = size / 2;
+    float best = sah_inf();
+    for (int a = 0; a < 3; ++a) {
+        if (scale[a] <= 0.f) continue;  // (warp-uniform)
+        int32_t L[kSahBinWords], R[kSahBinWords];
+        const int32_t *w = bins + (a * kSahBins + lane) * kSahBinWords;
+#pragma unroll
+        for (int j = 0; j < kSahBinWords; ++j) L[j] = R[j] = w[j];
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            int32_t u[kSahBinWords], d[kSahBinWords];
+#pragma unroll
+            for (int j = 0; j < kSahBinWords; ++j) { u[j] = __shfl_up_sync(0xffffffffu, L[j], off); d[j] = __shfl_down_sync(0xffffffffu, R[j], off); }
+            if (lane >= off) sah_bin_merge(L, u);
+            if (lane + off < 32) sah_bin_merge(R, d);
+        }
+        int32_t R1[kSahBinWords];
+#pragma unroll
+        for (int j = 0; j < kSahBinWords; ++j) R1[j] = __shfl_down_sync(0xffffffffu, R[j], 1);
+        const float c = lane + 1 < kSahBins ? sah_plane_cost(L, R1) : sah_inf();
+        const unsigned cb = __float_as_uint(c);  // (c >= 0: the bits order as the values)
+        const unsigned m = __reduce_min_sync(0xffffffffu, cb);
+        const int k = __ffs(__ballot_sync(0xffffffffu, cb == m)) - 1;
+        const int nl = __shfl_sync(0xffffffffu, L[0], k);
+        if (__uint_as_float(m) < best) { best = __uint_as_float(m); s.axis = a; s.plane = k; s.nl = nl; }
+    }
+    return s;
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_bounds(SahArgs a) {
+    __shared__ int32_t part[kSahBlock / 32][12];
+    int t, p0, p1;
+    if (!sah_block_range(a, t, p0, p1)) return;
+    int32_t b[12];
+    sah_bnd_init(b);
+    for (int p = p0 + threadIdx.x; p < p1; p += kSahBlock) { const int g = a.idx[p]; sah_bnd_add(b, a.prim_lo[g], a.prim_hi[g]); }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < 12; ++k) b[k] = (k % 6) < 3 ? __reduce_min_sync(0xffffffffu, b[k]) : __reduce_max_sync(0xffffffffu, b[k]);
+    if ((threadIdx.x & 31) == 0)
+        for (int k = 0; k < 12; ++k) part[threadIdx.x >> 5][k] = b[k];
+    __syncthreads();
+    if (threadIdx.x < 12) {
+        const int k = threadIdx.x;
+        int32_t v = part[0][k];
+        for (int w = 1; w < kSahBlock / 32; ++w) v = (k % 6) < 3 ? min(v, part[w][k]) : max(v, part[w][k]);
+        if ((k % 6) < 3) atomicMin(&a.tin[t].bnd[k], v); else atomicMax(&a.tin[t].bnd[k], v);
+    }
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_bin(SahArgs a) {
+    __shared__ int32_t bins[kSahBinsWords];
+    int t, p0, p1;
+    if (!sah_block_range(a, t, p0, p1)) return;
+    int32_t bnd[12]; float scale[3];
+    sah_load_bnd(a.tin_c[t], bnd, scale);
+    if (!(scale[0] > 0.f || scale[1] > 0.f || scale[2] > 0.f)) return;  // split by position: no bins
+    for (int k = threadIdx.x; k < 3 * kSahBins; k += kSahBlock) sah_bin_init(bins + k * kSahBinWords);
+    __syncthreads();
+    for (int p = p0 + threadIdx.x; p < p1; p += kSahBlock) { const int g = a.idx[p]; sah_bin_add(bins, a.prim_lo[g], a.prim_hi[g], bnd, scale); }
+    __syncthreads();
+    int32_t *dst = a.bins + (size_t)t * kSahBinsWords;
+    for (int k = threadIdx.x; k < 3 * kSahBins; k += kSahBlock) {
+        const int32_t *w = bins + k * kSahBinWords;
+        if (w[0] == 0) continue;
+        int32_t *d = dst + k * kSahBinWords;
+        atomicAdd(d, w[0]);
+        for (int j = 0; j < 3; ++j) { atomicMin(d + 1 + j, w[1 + j]); atomicMax(d + 4 + j, w[4 + j]); }
+    }
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_split(SahArgs a) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) { *a.n_clear = 0; *a.n_blk_clear = 0; }
+    const int t = (blockIdx.x * kSahBlock + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (t >= *a.n_tin) return;  // (warp-uniform)
+    SahTask &T = a.tin[t];
+    int32_t bnd[12]; float scale[3];
+    sah_load_bnd(T, bnd, scale);
+    int32_t *bins = a.bins + (size_t)t * kSahBinsWords;
+    const SahSplit s = sah_choose_warp(bins, scale, T.r.end - T.r.begin, lane);
+    __syncwarp();
+    for (int k = lane; k < 3 * kSahBins; k += 32) sah_bin_init(bins + k * kSahBinWords);  // neutral for the next level
+    if (lane == 0) {
+        T.axis = s.axis; T.plane = s.plane; T.nl = s.nl;
+        SahRange ch[2];
+        sah_make_node(a, T.r, bnd, s.nl, a.node_counter, ch);
+        sah_push_child(a, ch[0]); sah_push_child(a, ch[1]);
+    }
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_flag(SahArgs a) {
+    int t, p0, p1;
+    if (!sah_block_range(a, t, p0, p1)) return;
+    const SahTask &T = a.tin_c[t];
+    int32_t bnd[12]; float scale[3];
+    sah_load_bnd(T, bnd, scale);
+    SahSplit s; s.axis = T.axis; s.plane = T.plane; s.nl = T.nl;
+    for (int p = p0 + threadIdx.x; p < p1; p += kSahBlock) {
+        const int g = a.idx[p];
+        a.flags[p] = sah_goes_left(s, p - T.r.begin, a.prim_lo[g], a.prim_hi[g], bnd) ? 1 : 0;
+    }
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_scatter(SahArgs a) {
+    int t, p0, p1;
+    if (!sah_block_range(a, t, p0, p1)) return;
+    const SahTask &T = a.tin_c[t];
+    const int b = T.r.begin, nl = T.nl, base = a.scan[b];
+    for (int p = p0 + threadIdx.x; p < p1; p += kSahBlock) {
+        const int before = a.scan[p] - base;  // left-goers in [b, p)
+        a.idx2[a.flags[p] ? b + before : b + nl + (p - b - before)] = a.idx[p];
+    }
+}
+__global__ void __launch_bounds__(kSahBlock) k_sah_copy(SahArgs a) {
+    int t, p0, p1;
+    if (!sah_block_range(a, t, p0, p1)) return;
+    for (int p = p0 + threadIdx.x; p < p1; p += kSahBlock) a.idx[p] = a.idx2[p];
+}
+// The ranges of <= kSahSmall primitives, one block each: boxes and positions in shared memory, the subtree level by
+// level inside the block, one warp per range of a level (the rule of the large levels: same bounds, bins, choice and
+// stable partition).  Inner ids: one atomic per block for the whole subtree.
+constexpr int kSahSmallWarps = 8;
+struct SahSmallSmem {
+    float box[6][kSahSmall];  // lo xyz, hi xyz of local primitive slot
+    int32_t gidx[kSahSmall], slot[kSahSmall], scratch[kSahSmall];  // slot at each position of the range, partition buffer
+    SahRange list[2][kSahSmall / 2];
+    int32_t bins[kSahSmallWarps][kSahBinsWords];
+    int32_t n_cur, n_next, ids;
+};
+__device__ __forceinline__ void sah_small_box(const SahSmallSmem &S, int sl, F4 &lo, F4 &hi) {
+    lo.x = S.box[0][sl]; lo.y = S.box[1][sl]; lo.z = S.box[2][sl]; lo.w = 0.f;
+    hi.x = S.box[3][sl]; hi.y = S.box[4][sl]; hi.z = S.box[5][sl]; hi.w = 0.f;
+}
+__device__ void sah_small_range(const SahArgs &a, SahSmallSmem &S, const SahRange r, int B, int lane, int warp, int nxt) {
+    const int b = r.begin - B, e = r.end - B;
+    int32_t bnd[12];
+    sah_bnd_init(bnd);
+    for (int j = b + lane; j < e; j += 32) { F4 lo, hi; sah_small_box(S, S.slot[j], lo, hi); sah_bnd_add(bnd, lo, hi); }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < 12; ++k) bnd[k] = (k % 6) < 3 ? __reduce_min_sync(0xffffffffu, bnd[k]) : __reduce_max_sync(0xffffffffu, bnd[k]);
+    float scale[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) scale[k] = sah_scale(bnd, k);
+    int32_t *bins = S.bins[warp];
+    for (int k = lane; k < 3 * kSahBins; k += 32) sah_bin_init(bins + k * kSahBinWords);
+    __syncwarp();
+    if (scale[0] > 0.f || scale[1] > 0.f || scale[2] > 0.f)
+        for (int j = b + lane; j < e; j += 32) { F4 lo, hi; sah_small_box(S, S.slot[j], lo, hi); sah_bin_add(bins, lo, hi, bnd, scale); }
+    __syncwarp();
+    const SahSplit s = sah_choose_warp(bins, scale, e - b, lane);
+    int nl_seen = 0, nr_seen = 0;
+    const unsigned below = (1u << lane) - 1u;
+    for (int base = b; base < e; base += 32) {  // (warp-uniform)
+        const int j = base + lane;
+        const bool in = j < e;
+        const int sl = in ? S.slot[j] : 0;
+        F4 lo, hi;
+        sah_small_box(S, sl, lo, hi);
+        const bool f = in && sah_goes_left(s, j - b, lo, hi, bnd);
+        const unsigned lm = __ballot_sync(0xffffffffu, f), rm = __ballot_sync(0xffffffffu, in && !f);
+        if (f) S.scratch[b + nl_seen + __popc(lm & below)] = sl;
+        else if (in) S.scratch[b + s.nl + nr_seen + __popc(rm & below)] = sl;
+        nl_seen += __popc(lm); nr_seen += __popc(rm);
+    }
+    __syncwarp();
+    for (int j = b + lane; j < e; j += 32) S.slot[j] = S.scratch[j];
+    __syncwarp();
+    if (lane == 0) {
+        SahRange ch[2];
+        sah_make_node(a, r, bnd, s.nl, &S.ids, ch);
+        for (int k = 0; k < 2; ++k)
+            if (ch[k].end - ch[k].begin > 1) S.list[nxt][atomicAdd(&S.n_next, 1)] = ch[k];
+    }
+    __syncwarp();
+}
+__global__ void __launch_bounds__(kSahSmallWarps * 32) k_sah_small(SahArgs a) {
+    extern __shared__ __align__(16) unsigned char sah_smem[];
+    SahSmallSmem &S = *reinterpret_cast<SahSmallSmem *>(sah_smem);
+    const SahRange R = a.small[blockIdx.x];
+    const int B = R.begin, size = R.end - R.begin, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i < size; i += kSahSmallWarps * 32) {
+        const int g = a.idx[B + i];
+        const F4 lo = a.prim_lo[g], hi = a.prim_hi[g];
+        S.gidx[i] = g; S.slot[i] = i;
+        S.box[0][i] = lo.x; S.box[1][i] = lo.y; S.box[2][i] = lo.z; S.box[3][i] = hi.x; S.box[4][i] = hi.y; S.box[5][i] = hi.z;
+    }
+    if (tid == 0) {
+        S.list[0][0] = R; S.n_cur = 1;
+        S.ids = atomicAdd(a.node_counter, size - 2);  // ids of the subtree's size - 1 inner nodes but its root (R.id)
+    }
+    __syncthreads();
+    int cur = 0;
+    while (true) {  // one level of the subtree per pass; each pass splits every range in two, so sizes fall
+        const int m = S.n_cur;
+        if (m == 0) break;
+        if (tid == 0) S.n_next = 0;
+        __syncthreads();
+        for (int i = warp; i < m; i += kSahSmallWarps) sah_small_range(a, S, S.list[cur][i], B, lane, warp, cur ^ 1);
+        __syncthreads();
+        if (tid == 0) S.n_cur = S.n_next;
+        cur ^= 1;
+        __syncthreads();
+    }
+    for (int i = tid; i < size; i += kSahSmallWarps * 32) a.idx[B + i] = S.gidx[S.slot[i]];
+}
+
 // NCCL, loaded on first use.  A process that already holds a libnccl.so.2 (torch brings its own) gets that one.
 struct Nccl {
     void *lib = nullptr;
@@ -1018,6 +1244,27 @@ struct CudaBackend {
         ensure_temp(bytes);
         RTB_CUDA_CHECK(cub::DeviceSelect::If(cub_temp_, bytes, in, out, d_count, n, NonNegative(), stream_));
     }
+    // binned SAH: one level of large ranges (counts in device memory; grids cover the bounds) / all small ranges
+    void sah_level(const SahArgs &a, int block_bound, int task_bound) {
+        k_sah_bounds<<<block_bound, kSahBlock, 0, stream_>>>(a);
+        k_sah_bin<<<block_bound, kSahBlock, 0, stream_>>>(a);
+        k_sah_split<<<(task_bound * 32 + kSahBlock - 1) / kSahBlock, kSahBlock, 0, stream_>>>(a);
+        k_sah_flag<<<block_bound, kSahBlock, 0, stream_>>>(a);
+        RTB_CUDA_CHECK(cudaGetLastError());
+        size_t bytes = 0;
+        RTB_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, bytes, a.flags, a.scan, a.n, stream_));
+        ensure_temp(bytes);
+        RTB_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(cub_temp_, bytes, a.flags, a.scan, a.n, stream_));
+        k_sah_scatter<<<block_bound, kSahBlock, 0, stream_>>>(a);
+        k_sah_copy<<<block_bound, kSahBlock, 0, stream_>>>(a);
+        RTB_CUDA_CHECK(cudaGetLastError());
+    }
+    void sah_small(const SahArgs &a, int count) {
+        if (count <= 0) return;
+        RTB_CUDA_CHECK(cudaFuncSetAttribute(k_sah_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SahSmallSmem)));
+        k_sah_small<<<count, kSahSmallWarps * 32, sizeof(SahSmallSmem), stream_>>>(a);
+        RTB_CUDA_CHECK(cudaGetLastError());
+    }
     // one level of the collapse over the work items counted in device memory (k.a.n_in_dev): a resident grid strides
     // over them; *zero is cleared for the level after the next, *levels counts the levels that had work
     void collapse_level(const CollapseK &k, int bound, int32_t *zero, int32_t *levels) {
@@ -1050,6 +1297,8 @@ struct CudaBackend {
         return ms;
     }
 };
+
+static_assert(HasSahKernels<CudaBackend>::value, "the binned-SAH builder runs as k_sah_* kernels on the GPU");
 
 }  // namespace rtb
 

@@ -11,6 +11,7 @@
 // blocking 4-byte device->host copies per iteration); here an iteration is 4
 // launches (shade, generate, control, trace), and the host looks at one `done` word every few iterations.
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <stdexcept>
 #include <string>
@@ -474,8 +475,132 @@ struct RootItemK {  // the collapse starts from the root of the binary tree, whi
 // layout of the build's one block of counters (int32 unless noted): what the host reads back comes in ONE copy at the end
 enum BuildCtr {
     kCtrB2 = 0, kCtrWide = 1, kCtrTri = 2, kCtrNcl = 4, kCtrLevels = 5, kCtrLvl0 = 6 /* 6,7,8: work items of a level, rotating */,
-    kCtrSah = 9 /* float */, kCtrBounds = 16 /* 16..21 ordered floats, 22 = bad vertex */, kCtrTail = 24 /* 24: tail rounds, 25: root */, kCtrCount = 32
+    kCtrSah = 9 /* float */, kCtrSahTasks = 10 /* 10,11,12: large ranges of a level, rotating */,
+    kCtrSahBlocks = 13 /* 13,14,15: their blocks */, kCtrBounds = 16 /* 16..21 ordered floats, 22 = bad vertex */, kCtrTail = 24 /* 24: tail rounds, 25: root */,
+    kCtrSahSmall = 26 /* small ranges */, kCtrCount = 32
 };
+inline void check_builder(const rtb_build_params &bp) {
+    if (bp.builder != RTB_BUILDER_PLOC && bp.builder != RTB_BUILDER_BINNED_SAH) throw Error(RTB_ERR_INVALID, "unknown BVH builder");
+}
+struct SetK {
+    int32_t *p; int32_t v; int n;
+    RTB_HD void operator()(int i) const { if (i < n) p[i] = v; }
+};
+// RTB_BUILDER_BINNED_SAH: the binary tree (b2, count) over n >= 1 primitive boxes, its root in ctr[kCtrTail + 1].  Large
+// ranges are split level by level: the number of a level's ranges stays on the device (three rotating counters), the
+// host enqueues levels in batches and reads it once per batch; the ranges of <= kSahSmall primitives are finished
+// afterwards in one launch.  With `plan`, also the inner nodes deepest first (order) and where each depth starts in that
+// order (first[kSahMaxDepth + 1 - depth], -1 = no node of that depth; first[0]: deeper than kSahMaxDepth).
+// The binned-SAH steps as plain loops over the bodies of rtb_build.h, for a backend whose memory the host reads
+// directly (the host emulation that checks the builder without a GPU).  A backend with kernels of its own provides
+// sah_level / sah_small and is dispatched to them at compile time; rtb_cuda.cu asserts that CudaBackend does, so the
+// shipped library never reaches these loops.
+struct SahLoops {
+    // the split of one range from its bounds and bins, and the range partitioned stably: the kernels' rule
+    static SahSplit split(const SahArgs &a, const SahRange &r, int32_t *bnd) {
+        sah_bnd_init(bnd);
+        for (int p = r.begin; p < r.end; ++p) sah_bnd_add(bnd, a.prim_lo[a.idx[p]], a.prim_hi[a.idx[p]]);
+        const float scale[3] = {sah_scale(bnd, 0), sah_scale(bnd, 1), sah_scale(bnd, 2)};
+        std::vector<int32_t> bins(kSahBinsWords);
+        for (int k = 0; k < 3 * kSahBins; ++k) sah_bin_init(&bins[(size_t)k * kSahBinWords]);
+        for (int p = r.begin; p < r.end; ++p) sah_bin_add(bins.data(), a.prim_lo[a.idx[p]], a.prim_hi[a.idx[p]], bnd, scale);
+        const SahSplit s = sah_choose(bins.data(), scale, r.end - r.begin);
+        std::vector<int32_t> left, right;
+        for (int p = r.begin; p < r.end; ++p)
+            (sah_goes_left(s, p - r.begin, a.prim_lo[a.idx[p]], a.prim_hi[a.idx[p]], bnd) ? left : right).push_back(a.idx[p]);
+        if ((int)left.size() != s.nl) throw Error(RTB_ERR_INVALID, "internal: binned SAH partition disagrees with its bins");
+        std::copy(left.begin(), left.end(), a.idx + r.begin);
+        std::copy(right.begin(), right.end(), a.idx + r.begin + s.nl);
+        return s;
+    }
+    static void level(const SahArgs &a) {
+        *a.n_clear = 0; *a.n_blk_clear = 0;
+        for (int t = 0; t < *a.n_tin; ++t) {
+            SahTask &T = a.tin[t];
+            const SahSplit s = split(a, T.r, T.bnd);
+            SahRange ch[2];
+            sah_make_node(a, T.r, T.bnd, s.nl, a.node_counter, ch);
+            sah_push_child(a, ch[0]); sah_push_child(a, ch[1]);
+        }
+    }
+    static void subtree(const SahArgs &a, const SahRange &r) {
+        int32_t bnd[12];
+        const SahSplit s = split(a, r, bnd);
+        SahRange ch[2];
+        sah_make_node(a, r, bnd, s.nl, a.node_counter, ch);
+        for (const SahRange &c : ch) if (c.end - c.begin > 1) subtree(a, c);
+    }
+};
+template <class BE, class = void> struct HasSahKernels : std::false_type {};
+template <class BE>
+struct HasSahKernels<BE, std::void_t<decltype(std::declval<BE &>().sah_small(std::declval<const SahArgs &>(), 0))>> : std::true_type {};
+template <class BE>
+void sah_level(BE &be, const SahArgs &a, int block_bound, int task_bound) {
+    if constexpr (HasSahKernels<BE>::value) be.sah_level(a, block_bound, task_bound);
+    else SahLoops::level(a);
+}
+template <class BE>
+void sah_small(BE &be, const SahArgs &a, int count) {
+    if constexpr (HasSahKernels<BE>::value) be.sah_small(a, count);
+    else for (int i = 0; i < count; ++i) SahLoops::subtree(a, a.small[i]);
+}
+struct SahOrder { const int32_t *order = nullptr, *first = nullptr; };
+template <class BE>
+SahOrder build_binned_sah(BE &be, Temps<BE> &tmp, int n, const F4 *prim_lo, const F4 *prim_hi, B2Node *b2, int32_t *count,
+                          int32_t *ctr, bool plan) {
+    SahArgs a{};
+    a.prim_lo = prim_lo; a.prim_hi = prim_hi; a.n = n;
+    a.nodes = b2; a.count = count; a.node_counter = ctr + kCtrB2; a.n_small = ctr + kCtrSahSmall;
+    a.idx = tmp.template alloc<int32_t>(n); a.idx2 = tmp.template alloc<int32_t>(n);
+    a.flags = tmp.template alloc<int32_t>(n); a.scan = tmp.template alloc<int32_t>(n);
+    a.depth = tmp.template alloc<int32_t>(n > 1 ? n - 1 : 1);
+    const int task_bound = n / (kSahSmall + 1) + 1, block_bound = n / kSahChunk + task_bound;
+    SahTask *tasks[2] = {tmp.template alloc<SahTask>(task_bound), tmp.template alloc<SahTask>(task_bound)};
+    int32_t *blocks[2] = {tmp.template alloc<int32_t>(block_bound), tmp.template alloc<int32_t>(block_bound)};
+    a.bins = tmp.template alloc<int32_t>((size_t)task_bound * kSahBinsWords);
+    a.small = tmp.template alloc<SahRange>(n / 2 + 1);
+    { SahIotaK k; k.p = a.idx; k.n = n; be.launch(n, k); }
+    be.zero(a.flags, (size_t)n);
+    { SahBinsInitK k; k.bins = a.bins; k.n = task_bound * 3 * kSahBins; be.launch(k.n, k); }
+    // level L reads tasks[L & 1] and the counters at L % 3, writes tasks[(L + 1) & 1] and the counters at (L + 1) % 3,
+    // and clears those at (L + 2) % 3 for the level after the next
+    auto level_args = [&](int L) {
+        SahArgs l = a;
+        l.tin = tasks[(L + 2) & 1]; l.tin_c = l.tin; l.tout = tasks[(L + 3) & 1];
+        l.blk_in = blocks[(L + 2) & 1]; l.blk_out = blocks[(L + 3) & 1];
+        l.n_tin = ctr + kCtrSahTasks + (L + 3) % 3; l.n_tout = ctr + kCtrSahTasks + (L + 4) % 3; l.n_clear = ctr + kCtrSahTasks + (L + 5) % 3;
+        l.n_blk_in = ctr + kCtrSahBlocks + (L + 3) % 3; l.n_blk_out = ctr + kCtrSahBlocks + (L + 4) % 3;
+        l.n_blk_clear = ctr + kCtrSahBlocks + (L + 5) % 3;
+        return l;
+    };
+    { SahRootK r; r.a = level_args(-1); r.root = ctr + kCtrTail + 1; be.launch(1, r); }  // (the root is level 0's one range)
+    int level = 0;
+    int32_t pending = n > kSahSmall ? 1 : 0;
+    while (pending > 0) {
+        for (int b = 0; b < 4; ++b, ++level) sah_level(be, level_args(level), block_bound, task_bound);
+        be.download(&pending, ctr + kCtrSahTasks + level % 3, 1);
+        // (ranges of level L are at depth >= L: the loop ends, with a tree or with this error)
+        if (pending > 0 && level > kSahMaxDepth) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+    }
+    int32_t n_small = 0;
+    be.download(&n_small, a.n_small, 1);
+    sah_small(be, a, n_small);
+    { SahLeafK k; k.a = a; be.launch(n, k); }
+    tmp.free(a.idx); tmp.free(a.idx2); tmp.free(a.flags); tmp.free(a.scan); tmp.free(tasks[0]); tmp.free(tasks[1]);
+    tmp.free(blocks[0]); tmp.free(blocks[1]); tmp.free(a.bins); tmp.free(a.small);
+    SahOrder o;
+    if (!plan || n < 2) return o;
+    const int n_inner = n - 1;
+    uint64_t *keys = tmp.template alloc<uint64_t>(n_inner);
+    int32_t *order = tmp.template alloc<int32_t>(n_inner), *first = tmp.template alloc<int32_t>(kSahMaxDepth + 2);
+    { SahDepthKeyK k; k.depth = a.depth; k.keys = keys; k.vals = order; k.n_inner = n_inner; k.n = n; be.launch(n_inner, k); }
+    be.sort_pairs(keys, order, n_inner);
+    { SetK k; k.p = first; k.v = -1; k.n = kSahMaxDepth + 2; be.launch(k.n, k); }
+    { SahGroupK k; k.keys = keys; k.first = first; k.n_inner = n_inner; be.launch(n_inner, k); }
+    tmp.free(keys);
+    o.order = order; o.first = first;
+    return o;
+}
 constexpr int kMaxPlocLog = 1 << 16;
 template <class BE>
 BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriMeta *meta_in, const F4 *box_lo, const F4 *box_hi,
@@ -483,8 +608,6 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
                      int32_t *leaf_of_prim) {
     BuiltTree out;
     Temps<BE> tmp(be);
-    if (bp.builder != RTB_BUILDER_PLOC) throw Error(RTB_ERR_INVALID, "unknown BVH builder");
-    const int radius = bp.ploc_radius > 0 ? bp.ploc_radius : 16;
     // 1. per-triangle records, bounds
     F4 *prim_lo = tmp.template alloc<F4>(n), *prim_hi = tmp.template alloc<F4>(n);
     int32_t *ctr = tmp.template alloc<int32_t>(kCtrCount);
@@ -512,63 +635,16 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
             }
         }
     }
-    // 2. Morton codes + sort
-    uint64_t *keys = tmp.template alloc<uint64_t>(n);
-    int32_t *sorted = tmp.template alloc<int32_t>(n);
-    {
-        MortonK k; k.a.prim_lo = prim_lo; k.a.prim_hi = prim_hi; k.a.scene_bounds = bounds; k.a.keys = keys; k.a.vals = sorted; k.a.n = n;
-        be.launch(n, k);
-        be.sort_pairs(keys, sorted, n);
-    }
-    // 3. PLOC.  The cluster count stays on the device (ctr[kCtrNcl]); the host enqueues a batch of rounds against an
-    // upper bound of it and reads the count back once per batch (round 1: after every round).
     const int n_b2 = 2 * n - 1;
     B2Node *b2 = tmp.template alloc<B2Node>(n_b2);
     int32_t *count = tmp.template alloc<int32_t>(n_b2);
-    int32_t *ca = tmp.template alloc<int32_t>(n), *cb = tmp.template alloc<int32_t>(n), *nn = tmp.template alloc<int32_t>(n);
     const bool want_plan = bp.collapse == RTB_COLLAPSE_SAH_OPTIMAL && n > max_leaf;
-    int32_t *log = tmp.template alloc<int32_t>(kMaxPlocLog);
-    {
-        PlocLeafK k; k.lo = prim_lo; k.hi = prim_hi; k.sorted = sorted; k.nodes = b2; k.count = count; k.clusters = ca; k.n = n;
-        be.launch(n, k);
-    }
-    int bound = n, rounds = 0;
-    bool tail = false;
-    while (bound > 1) {
-        PlocArgs a; a.nodes = b2; a.count = count; a.cin = ca; a.cout = cb; a.nn = nn; a.node_counter = ctr + kCtrB2; a.ncl = bound; a.radius = radius;
-        a.ncl_dev = ctr + kCtrNcl; a.log = log; a.round = rounds;
-        // the last rounds handle a few hundred clusters each and are pure launch latency (S1: 28 of 46 rounds): once
-        // the clusters fit one thread block, one launch runs all the remaining rounds in shared memory
-        if (be.ploc_tail(a, n, ctr + kCtrTail)) { tail = true; break; }
-        // rounds of this batch: the count shrinks by about a fifth per round (S1 and S2 alike); go most of the way to
-        // the tail's size, but not far on a large bound — every launch of the batch still covers the whole bound
-        const double to_tail = std::log((double)bound / 1024.0) / 0.235;
-        int batch = (int)(0.8 * to_tail);
-        const int cap = bound > (1 << 21) ? 4 : (bound > (1 << 18) ? 8 : 16);
-        if (batch > cap) batch = cap;
-        if (batch < 1) batch = 1;
-        for (int r = 0; r < batch; ++r) {
-            // (a scene of identical triangles merges ONE pair per round: n - 1 rounds.  The per-round counts are a
-            // statistic, and the SAH-optimal plan's launch schedule: beyond the log's size only the plan needs them)
-            if (rounds >= kMaxPlocLog) {
-                if (want_plan) throw Error(RTB_ERR_INVALID, "RTB_COLLAPSE_SAH_OPTIMAL: too many PLOC rounds (degenerate scene)");
-                a.log = nullptr;
-            }
-            a.round = rounds;
-            be.ploc_nn(a);
-            PlocMergeK k2; k2.a = a; k2.n_leaves = n; be.launch(bound, k2);
-            be.compact_nonneg(cb, ca, bound, ctr + kCtrNcl);
-            ++rounds;
-        }
-        int32_t now = 0;
-        be.download(&now, ctr + kCtrNcl, 1);
-        if (now >= bound) throw Error(RTB_ERR_INVALID, "internal: a PLOC round merged nothing");  // (cannot happen with finite boxes: the lowest-area pair is mutual)
-        bound = now;
-    }
-    tmp.free(prim_lo); tmp.free(prim_hi); tmp.free(keys); tmp.free(sorted); tmp.free(nn);
-    // 4. collapse plan: bottom-up over the binary tree, one launch per PLOC round (a round's nodes only have older children)
     float *plan_cost = nullptr; uint8_t *plan = nullptr;
+    const int32_t *root_src = ctr + kCtrTail + 1;
+    int rounds = 0;
+    bool tail = false;
     std::vector<int32_t> hlog, htail;
+    int32_t *log = nullptr;
     auto read_logs = [&]() {
         const int logged = rounds < kMaxPlocLog ? rounds : kMaxPlocLog;
         hlog.resize((size_t)logged + 1);
@@ -582,21 +658,96 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
             if (h2[0]) be.download(htail.data(), be.ploc_tail_counts(), (size_t)h2[0]);
         }
     };
-    if (want_plan) {
-        read_logs();
-        plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
-        plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
-        int next_id = n;
-        auto plan_round = [&](int made) {
-            if (made > 0) {
-                PlanK k; k.a.nodes = b2; k.a.count = count; k.a.cost = plan_cost; k.a.plan = plan;
-                k.a.first = next_id; k.a.n = made; k.a.max_leaf = max_leaf;
-                be.launch(made, k);
+    if (bp.builder == RTB_BUILDER_PLOC) {
+        const int radius = bp.ploc_radius > 0 ? bp.ploc_radius : 16;
+        // 2. Morton codes + sort
+        uint64_t *keys = tmp.template alloc<uint64_t>(n);
+        int32_t *sorted = tmp.template alloc<int32_t>(n);
+        {
+            MortonK k; k.a.prim_lo = prim_lo; k.a.prim_hi = prim_hi; k.a.scene_bounds = bounds; k.a.keys = keys; k.a.vals = sorted; k.a.n = n;
+            be.launch(n, k);
+            be.sort_pairs(keys, sorted, n);
+        }
+        // 3. PLOC.  The cluster count stays on the device (ctr[kCtrNcl]); the host enqueues a batch of rounds against an
+        // upper bound of it and reads the count back once per batch (round 1: after every round).
+        int32_t *ca = tmp.template alloc<int32_t>(n), *cb = tmp.template alloc<int32_t>(n), *nn = tmp.template alloc<int32_t>(n);
+        log = tmp.template alloc<int32_t>(kMaxPlocLog);
+        {
+            PlocLeafK k; k.lo = prim_lo; k.hi = prim_hi; k.sorted = sorted; k.nodes = b2; k.count = count; k.clusters = ca; k.n = n;
+            be.launch(n, k);
+        }
+        int bound = n;
+        while (bound > 1) {
+            PlocArgs a; a.nodes = b2; a.count = count; a.cin = ca; a.cout = cb; a.nn = nn; a.node_counter = ctr + kCtrB2; a.ncl = bound; a.radius = radius;
+            a.ncl_dev = ctr + kCtrNcl; a.log = log; a.round = rounds;
+            // the last rounds handle a few hundred clusters each and are pure launch latency (S1: 28 of 46 rounds): once
+            // the clusters fit one thread block, one launch runs all the remaining rounds in shared memory
+            if (be.ploc_tail(a, n, ctr + kCtrTail)) { tail = true; break; }
+            // rounds of this batch: the count shrinks by about a fifth per round (S1 and S2 alike); go most of the way to
+            // the tail's size, but not far on a large bound — every launch of the batch still covers the whole bound
+            const double to_tail = std::log((double)bound / 1024.0) / 0.235;
+            int batch = (int)(0.8 * to_tail);
+            const int cap = bound > (1 << 21) ? 4 : (bound > (1 << 18) ? 8 : 16);
+            if (batch > cap) batch = cap;
+            if (batch < 1) batch = 1;
+            for (int r = 0; r < batch; ++r) {
+                // (a scene of identical triangles merges ONE pair per round: n - 1 rounds.  The per-round counts are a
+                // statistic, and the SAH-optimal plan's launch schedule: beyond the log's size only the plan needs them)
+                if (rounds >= kMaxPlocLog) {
+                    if (want_plan) throw Error(RTB_ERR_INVALID, "RTB_COLLAPSE_SAH_OPTIMAL: too many PLOC rounds (degenerate scene)");
+                    a.log = nullptr;
+                }
+                a.round = rounds;
+                be.ploc_nn(a);
+                PlocMergeK k2; k2.a = a; k2.n_leaves = n; be.launch(bound, k2);
+                be.compact_nonneg(cb, ca, bound, ctr + kCtrNcl);
+                ++rounds;
             }
-            next_id += made;
-        };
-        for (size_t r = 0; r + 1 < hlog.size(); ++r) plan_round(hlog[r] - hlog[r + 1]);
-        for (int32_t c : htail) plan_round(c);
+            int32_t now = 0;
+            be.download(&now, ctr + kCtrNcl, 1);
+            if (now >= bound) throw Error(RTB_ERR_INVALID, "internal: a PLOC round merged nothing");  // (cannot happen with finite boxes: the lowest-area pair is mutual)
+            bound = now;
+        }
+        if (!tail) root_src = ca;
+        tmp.free(prim_lo); tmp.free(prim_hi); tmp.free(keys); tmp.free(sorted); tmp.free(nn);
+        // 4. collapse plan: bottom-up over the binary tree, one launch per PLOC round (a round's nodes only have older children)
+        if (want_plan) {
+            read_logs();
+            plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
+            plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
+            int next_id = n;
+            auto plan_round = [&](int made) {
+                if (made > 0) {
+                    PlanK k; k.a.nodes = b2; k.a.count = count; k.a.cost = plan_cost; k.a.plan = plan;
+                    k.a.first = next_id; k.a.n = made; k.a.max_leaf = max_leaf; k.a.order = nullptr;
+                    be.launch(made, k);
+                }
+                next_id += made;
+            };
+            for (size_t r = 0; r + 1 < hlog.size(); ++r) plan_round(hlog[r] - hlog[r + 1]);
+            for (int32_t c : htail) plan_round(c);
+        }
+    } else {
+        // 2'-3'. binned SAH, top down; the root goes to ctr[kCtrTail + 1]
+        const SahOrder so = build_binned_sah(be, tmp, n, prim_lo, prim_hi, b2, count, ctr, want_plan);
+        const int32_t *order = so.order;
+        tmp.free(prim_lo); tmp.free(prim_hi);
+        // 4. collapse plan: one launch per depth, deepest first (a node's children are deeper)
+        if (want_plan) {
+            std::vector<int32_t> first(kSahMaxDepth + 2);
+            be.download(first.data(), so.first, first.size());  // (the one read-back of the per-depth counts)
+            if (first[0] >= 0) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+            plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
+            plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
+            for (int k = 1; k <= kSahMaxDepth + 1; ++k) {
+                if (first[(size_t)k] < 0) continue;
+                int end = n - 1;
+                for (int j = k + 1; j <= kSahMaxDepth + 1; ++j) if (first[(size_t)j] >= 0) { end = first[(size_t)j]; break; }
+                PlanK p; p.a.nodes = b2; p.a.count = count; p.a.cost = plan_cost; p.a.plan = plan;
+                p.a.first = first[(size_t)k]; p.a.n = end - first[(size_t)k]; p.a.max_leaf = max_leaf; p.a.order = order;
+                be.launch(p.a.n, p);
+            }
+        }
     }
     // 5. collapse to the 8-wide compressed tree, level by level; the number of work items of a level stays on the
     // device (three rotating counters: read, written, cleared), the host reads it once per batch of levels
@@ -606,7 +757,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
     int32_t *gather = tmp.template alloc<int32_t>(n);
     CollapseArgs ga{};
     {
-        RootItemK r; r.root_src = tail ? ctr + kCtrTail + 1 : ca; r.dst = wa;
+        RootItemK r; r.root_src = root_src; r.dst = wa;
         be.launch(1, r);
     }
     int level = 0;
@@ -636,7 +787,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
     if (c[kCtrTri] != n) throw Error(RTB_ERR_INVALID, "internal: collapse lost triangles");
     out.nodes8 = be.template alloc<Q4>((size_t)out.num_nodes * kNodeWords);
     be.copy(out.nodes8, nodes_tmp, (size_t)out.num_nodes * kNodeWords);
-    if (!want_plan) read_logs();
+    if (bp.builder == RTB_BUILDER_PLOC && !want_plan) read_logs();
     int iters = rounds > kMaxPlocLog ? rounds - kMaxPlocLog : 0;  // (rounds beyond the log are counted, not examined)
     for (size_t r = 0; r + 1 < hlog.size(); ++r) if (hlog[r] > hlog[r + 1]) ++iters;
     out.ploc_iterations = iters + (int)htail.size();
@@ -658,7 +809,7 @@ void build_bvh(BE &be, SceneT<BE> &sc, const float *d_vertices, Tri48 *tri_in, T
     const int64_t n64 = sc.n;
     if (n64 > 0x3fffffff) throw Error(RTB_ERR_INVALID, "too many triangles (max 2^30-1)");
     const int n = (int)n64;
-    if (bp.builder != RTB_BUILDER_PLOC) throw Error(RTB_ERR_INVALID, "unknown BVH builder");
+    check_builder(bp);
     const int max_leaf = bp.max_leaf_tris >= 1 && bp.max_leaf_tris <= 3 ? bp.max_leaf_tris : 3;
     auto t0 = be.now();
     sc.stats = rtb_bvh_stats{};
@@ -1001,7 +1152,7 @@ SceneT<BE> *scene_from_instanced(BE &be, const rtb_instanced_scene_desc &D, cons
         o.Lx = l.L[0]; o.Ly = l.L[1]; o.Lz = l.L[2];
         light_tri[(size_t)i] = l.type == RTB_AREA_LIGHT ? l.triangle : 0;
     }
-    if (bp.builder != RTB_BUILDER_PLOC) throw Error(RTB_ERR_INVALID, "unknown BVH builder");
+    check_builder(bp);
     const int max_leaf = bp.max_leaf_tris >= 1 && bp.max_leaf_tris <= 3 ? bp.max_leaf_tris : 3;
     SceneT<BE> *sc = new SceneT<BE>();
     std::vector<BuiltTree> trees((size_t)nm);

@@ -30,6 +30,7 @@ ap.add_argument("--device", type=int, default=0)
 ap.add_argument("--radius", type=int, default=0)
 ap.add_argument("--leaf", type=int, default=0)
 ap.add_argument("--collapse", type=int, default=-1)
+ap.add_argument("--builder", type=int, default=-1, help="rtb_build_params.builder (0 PLOC, 1 binned SAH)")
 ap.add_argument("--count", action="store_true", help="also print nodes / triangles per ray (counting kernels)")
 ap.add_argument("--reps", type=int, default=2)
 ap.add_argument("--flags", type=int, default=0)
@@ -48,6 +49,7 @@ for refill, chunk, pool, pooled, fused, pf, pipes in itertools.product(a.refill.
     if a.radius: bp.ploc_radius = a.radius
     if a.leaf: bp.max_leaf_tris = a.leaf
     if a.collapse >= 0: bp.collapse = a.collapse
+    if a.builder >= 0: bp.builder = a.builder
     sc = ctx.scene(hs.desc, bp)
     bs = sc.stats()
     p = capi.render_params(L, width=w, height=h, spp=spp, max_bounces=depth, flags=a.flags, first_sample=a.first_sample, total_spp=spp + a.first_sample)
