@@ -135,6 +135,14 @@ enum {
                                    is 0.  Exact-t ties at shared edges can resolve differently from the reference, as
                                    with RTB_COLLAPSE_SAH_OPTIMAL (DESIGN.md 4.1) */
 };
+/* Treelet restructuring of the binary tree after the builder, k = 0..8 passes, or-ed into the builder value:
+   bp.builder = RTB_BUILDER_PLOC | RTB_BUILDER_TREELET_PASSES(3).  One pass visits the inner nodes bottom-up; each node
+   with enough triangles below it (7 in the first pass, doubling with every pass) is the root of a treelet of up to 7
+   subtrees, which is rewired into the binary topology over them with the lowest total surface area (Karras & Aila
+   2013).  Works with both builders and both collapse modes; k = 0 is the plain builder.  Costs build time and gives a
+   lower SAH cost; exact-t ties at shared edges can resolve differently from the reference, as with
+   RTB_COLLAPSE_SAH_OPTIMAL (DESIGN.md 4.1).  Other bits of rtb_build_params.builder must be zero. */
+#define RTB_BUILDER_TREELET_PASSES(k) ((k) << 8)
 
 /* how the binary tree is collapsed into 8-wide nodes (rtb_build_params.collapse) */
 enum {
@@ -145,7 +153,7 @@ enum {
 };
 
 typedef struct rtb_build_params {
-    int32_t builder;      /* RTB_BUILDER_* */
+    int32_t builder;      /* RTB_BUILDER_*, | RTB_BUILDER_TREELET_PASSES(k) */
     int32_t ploc_radius;  /* nearest-neighbour search radius, 0 = default (16) */
     int32_t max_leaf_tris;/* 1..3, 0 = default (3) */
     int32_t collapse;     /* RTB_COLLAPSE_* */

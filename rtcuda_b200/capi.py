@@ -21,6 +21,13 @@ RTB_RENDER_PIXEL_CENTRE, RTB_RENDER_NO_SHADOW, RTB_RENDER_NONPERSISTENT, RTB_REN
 RTB_RENDER_SINGLE_PIPELINE = 16
 RTB_RENDER_TRUE_MIS, RTB_RENDER_RR_TERMINATE, RTB_RENDER_DETERMINISTIC = 32, 64, 128
 RTB_BUILDER_PLOC, RTB_BUILDER_BINNED_SAH = 0, 1
+
+
+def treelet_passes(k):
+    """RTB_BUILDER_TREELET_PASSES(k), k = 0..8: or it into the builder, e.g. RTB_BUILDER_PLOC | treelet_passes(3)"""
+    return k << 8
+
+
 RTB_COLLAPSE_LARGEST_FIRST, RTB_COLLAPSE_SAH_OPTIMAL = 0, 1
 
 

@@ -11,6 +11,10 @@
 //   3'. binned SAH    (RTB_BUILDER_BINNED_SAH, instead of 2-3) top-down
 //                     32-bin SAH splits down to single primitives: large
 //                     ranges level by level, small ones one block each
+//   3.5 treelets      (optional, RTB_BUILDER_TREELET_PASSES) passes of treelet
+//                     restructuring (Karras & Aila 2013) over either tree:
+//                     up to 7 subtrees under a node rewired into their
+//                     cheapest binary topology, one launch per depth
 //   4. collapse plan  (optional, RTB_COLLAPSE_SAH_OPTIMAL; default is the greedy
 //                     "largest child first" of step 5)
 //                     bottom-up dynamic programme over the binary tree (after
@@ -438,6 +442,188 @@ struct SahGroupK {
         if (i == 0 || keys[i - 1] != keys[i]) first[keys[i]] = i;
     }
 };
+
+// ------------------------------------------------------------ 3.5 treelet restructuring (RTB_BUILDER_TREELET_PASSES)
+// After either builder, on the binary tree in place (Karras & Aila 2013).  A pass visits the inner nodes deepest first,
+// one launch per depth; a node whose subtree holds at least gamma triangles is the root of a treelet: starting from its
+// two children, the treelet leaf with the largest area that is an inner node is opened (ties: the lower id) until 7
+// leaves or only leaves remain.  A dynamic programme over the subsets of those leaves finds the binary topology over
+// them with the lowest sum of inner node areas; when that sum is strictly lower than the present one, the treelet is
+// rewired with its own inner ids.  The leaves (their subtrees) stay as they are, the root keeps its id, and nodes of one
+// depth have disjoint subtrees, so a launch is free of races and its result does not depend on the schedule.  Costs
+// use the explicitly rounded arithmetic of plan_body: the GPU and the host emulation pick the same topologies.
+constexpr int kTloLeaves = 7;
+constexpr int kTloSubsets = 1 << kTloLeaves;
+constexpr int kTloMaxPasses = 8;  // RTB_BUILDER_TREELET_PASSES(k): k = 0..8
+// Pass p (from 0) restructures the treelets of nodes with at least kTloGamma << p triangles: later passes leave the
+// bottom of the tree, which the first pass already optimised, and cost a fraction of it.  (S1, 3 passes, both builders
+// and both collapses: 7 doubling comes within 0.04 % of the SAH cost of restructuring every treelet in every pass,
+// gamma 3; 14 doubling loses up to 0.1 % — DESIGN.md 4.1.)
+constexpr int kTloGamma = 7;
+struct TloArgs {
+    B2Node *nodes; int32_t *count;
+    int32_t *parent;          // [2n-1]: parent of every node, -1 at the root; kept up to date by the rewiring
+    int32_t *depth;           // [n-1]: depth of inner node id at [id - n], at most kSahMaxDepth + 1
+    const int32_t *root;      // the root's id (device memory)
+    const int32_t *order;     // inner nodes deepest first; this launch: roots order[first .. first + num)
+    int32_t first, num;
+    int32_t gamma, n;
+};
+// parents from the inner nodes (ids n .. 2n-2, whichever builder made them)
+struct TloParentK {
+    TloArgs a;
+    RTB_HD void operator()(int i) const {
+        if (i >= a.n - 1) return;
+        const B2Node x = a.nodes[a.n + i];
+        a.parent[x.left] = a.n + i; a.parent[x.right] = a.n + i;
+        if (i == 0) a.parent[*a.root] = -1;
+    }
+};
+// depth of every inner node by walking up to the root; a walk longer than kSahMaxDepth stops there (too deep anyway)
+struct TloDepthK {
+    TloArgs a;
+    RTB_HD void operator()(int i) const {
+        if (i >= a.n - 1) return;
+        int d = 0;
+        for (int p = a.parent[a.n + i]; p >= 0 && d <= kSahMaxDepth; p = a.parent[p]) ++d;
+        a.depth[i] = d;
+    }
+};
+// one treelet under work (shared memory on the GPU, one per warp): subsets are bit masks over the leaf slots
+struct TloWork {
+    float area[kTloSubsets];      // half area of the union of a subset's leaves
+    float cost[kTloSubsets];      // cheapest sum of inner areas over a subset (0 for one leaf)
+    uint8_t part[kTloSubsets];    // that topology's left child: the lowest mask of the cheapest partition
+    B2Node box[kTloLeaves];       // the leaves' nodes
+    int32_t leaf[kTloLeaves];     // their ids
+    int32_t lcount[kTloLeaves];   // and triangle counts
+    int32_t inner[kTloLeaves - 1];  // the treelet's inner ids: [0] the root, then in opening order
+    int32_t imask[kTloLeaves - 1]; float icost[kTloLeaves - 1];  // the present topology: leaves and cost of inner[j]
+    int32_t qmask[kTloLeaves - 1], qid[kTloLeaves - 1];          // the rewiring's queue
+    int32_t nl, ni;
+};
+RTB_HD void tlo_form(const TloArgs &a, TloWork &W, int root) {
+    const B2Node r = a.nodes[root];
+    W.inner[0] = root; W.ni = 1;
+    W.leaf[0] = r.left; W.box[0] = a.nodes[r.left];
+    W.leaf[1] = r.right; W.box[1] = a.nodes[r.right];
+    W.nl = 2;
+    const int32_t c0 = a.count[r.left], c1 = a.count[r.right];
+    W.lcount[0] = c0; W.lcount[1] = c1;
+    while (W.nl < kTloLeaves) {
+        int best = -1; float ba = 0.f;
+        for (int k = 0; k < W.nl; ++k) {
+            if (W.box[k].right < 0) continue;
+            const float ar = b2_half_area(W.box[k]);
+            if (best < 0 || ar > ba || (ar == ba && W.leaf[k] < W.leaf[best])) { best = k; ba = ar; }
+        }
+        if (best < 0) break;
+        const B2Node x = W.box[best];
+        W.inner[W.ni++] = W.leaf[best];
+        W.leaf[best] = x.left; W.box[best] = a.nodes[x.left]; W.lcount[best] = a.count[x.left];
+        W.leaf[W.nl] = x.right; W.box[W.nl] = a.nodes[x.right]; W.lcount[W.nl] = a.count[x.right];
+        ++W.nl;
+    }
+}
+// box (exact: min / max) and triangle count of the union of subset m
+RTB_HD B2Node tlo_union(const TloWork &W, int m, int &cnt) {
+    B2Node u; cnt = 0;
+    bool first = true;
+    for (int k = 0; k < W.nl; ++k) {
+        if (!(m >> k & 1)) continue;
+        const B2Node &b = W.box[k];
+        cnt += W.lcount[k];
+        if (first) { u = b; first = false; continue; }
+        u.lox = fminf(u.lox, b.lox); u.loy = fminf(u.loy, b.loy); u.loz = fminf(u.loz, b.loz);
+        u.hix = fmaxf(u.hix, b.hix); u.hiy = fmaxf(u.hiy, b.hiy); u.hiz = fmaxf(u.hiz, b.hiz);
+    }
+    return u;
+}
+// cost of subset m from those of its proper subsets: the partition {p, m ^ p} where p lacks m's highest leaf, so p is
+// the lower mask of the two; ties go to the lowest p
+RTB_HD void tlo_dp(TloWork &W, int m) {
+    int hb = m;
+    while (hb & (hb - 1)) hb &= hb - 1;
+    const int rest = m ^ hb;
+    if (rest == 0) { W.cost[m] = 0.f; W.part[m] = 0; return; }
+    float best = 0.f; int bp = -1;
+    for (int p = rest; p > 0; p = (p - 1) & rest) {  // (descending: `<=` keeps the lowest mask among equal costs)
+        const float v = fadd(W.cost[p], W.cost[m ^ p]);
+        if (bp < 0 || v <= best) { best = v; bp = p; }
+    }
+    W.cost[m] = fadd(W.area[m], best); W.part[m] = (uint8_t)bp;
+}
+// a child of inner[j] in the present topology: its leaf mask and cost (a leaf slot, or an inner node opened after j)
+RTB_HD void tlo_child(const TloWork &W, int id, int &mask, float &cost) {
+    for (int k = 0; k < W.nl; ++k) if (W.leaf[k] == id) { mask = 1 << k; cost = 0.f; return; }
+    for (int j = 1; j < W.ni; ++j) if (W.inner[j] == id) { mask = W.imask[j]; cost = W.icost[j]; return; }
+    mask = 0; cost = 0.f;  // (unreachable: every child of a treelet inner node is in the treelet)
+}
+// sum of inner areas of the present topology, with the programme's arithmetic (so the programme's cost is never higher)
+RTB_HD float tlo_present_cost(const TloArgs &a, TloWork &W) {
+    for (int j = W.ni - 1; j >= 0; --j) {  // (children were opened after their parent)
+        const B2Node x = a.nodes[W.inner[j]];
+        int ml, mr; float cl, cr;
+        tlo_child(W, x.left, ml, cl);
+        tlo_child(W, x.right, mr, cr);
+        W.imask[j] = ml | mr;
+        W.icost[j] = fadd(W.area[ml | mr], fadd(cl, cr));
+    }
+    return W.icost[0];
+}
+// the cheapest topology written over the treelet's inner ids: the root keeps its id, the other ids, in ascending
+// order, go to the new inner nodes in breadth-first order, left child first; boxes, counts and parents rewritten
+RTB_HD void tlo_rewrite(const TloArgs &a, TloWork &W, int full) {
+    for (int j = 2; j < W.ni; ++j)
+        for (int k = j; k > 1 && W.inner[k - 1] > W.inner[k]; --k) { const int t = W.inner[k]; W.inner[k] = W.inner[k - 1]; W.inner[k - 1] = t; }
+    int head = 0, tail = 0, next = 1;
+    W.qmask[tail] = full; W.qid[tail] = W.inner[0]; ++tail;
+    while (head < tail) {
+        const int m = W.qmask[head], id = W.qid[head];
+        ++head;
+        int ch[2];
+        for (int s = 0; s < 2; ++s) {
+            const int q = s == 0 ? W.part[m] : m ^ W.part[m];
+            if (q & (q - 1)) {
+                ch[s] = W.inner[next++];
+                W.qmask[tail] = q; W.qid[tail] = ch[s]; ++tail;
+            } else {
+                int k = 0;
+                while (!(q >> k & 1)) ++k;
+                ch[s] = W.leaf[k];
+            }
+        }
+        int cnt;
+        B2Node u = tlo_union(W, m, cnt);
+        u.left = ch[0]; u.right = ch[1];
+        a.nodes[id] = u;
+        a.count[id] = cnt;
+        a.parent[ch[0]] = id; a.parent[ch[1]] = id;
+    }
+}
+#if defined(__CUDA_ARCH__)
+#define RTB_TLO_SYNC() __syncwarp()
+#else
+#define RTB_TLO_SYNC()
+#endif
+// treelet of root order[first + tid], by `lanes` lanes (a warp on the GPU, 1 in the host emulation): lane 0 forms and
+// rewires it, the subsets are shared out between the lanes
+RTB_HD void tlo_treelet(const TloArgs &a, TloWork &W, int tid, int lane, int lanes) {
+    const int root = a.order[a.first + tid];
+    if (a.count[root] < a.gamma) return;
+    if (lane == 0) tlo_form(a, W, root);
+    RTB_TLO_SYNC();
+    const int nl = W.nl;
+    if (nl < 3) return;  // (two leaves: one topology)
+    const int full = (1 << nl) - 1;
+    for (int m = 1 + lane; m <= full; m += lanes) { int cnt; W.area[m] = b2_half_area(tlo_union(W, m, cnt)); }
+    RTB_TLO_SYNC();
+    for (int s = 1; s <= nl; ++s) {  // by subset size: a subset's partitions are smaller
+        for (int m = 1 + lane; m <= full; m += lanes) if (popc((uint32_t)m) == s) tlo_dp(W, m);
+        RTB_TLO_SYNC();
+    }
+    if (lane == 0 && W.cost[full] < tlo_present_cost(a, W)) tlo_rewrite(a, W, full);
+}
 
 // ------------------------------------------------------------ 4. collapse plan
 // cost[n][i-1], i = 1..7: SAH cost of subtree n laid out in at most i child

@@ -843,6 +843,18 @@ __global__ void __launch_bounds__(kSahSmallWarps * 32) k_sah_small(SahArgs a) {
     for (int i = tid; i < size; i += kSahSmallWarps * 32) a.idx[B + i] = S.gidx[S.slot[i]];
 }
 
+// ---- treelet restructuring (RTB_BUILDER_TREELET_PASSES, rtb_build.h 3.5) ----
+// One warp per treelet root of one depth: lane 0 forms the treelet and rewires it, the 32 lanes share the (<= 127)
+// subsets of the dynamic programme; the treelet's tables live in shared memory.
+constexpr int kTloWarps = 4;
+__global__ void __launch_bounds__(kTloWarps * 32) k_tlo_treelet(TloArgs a) {
+    __shared__ TloWork W[kTloWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int i = blockIdx.x * kTloWarps + warp;
+    if (i >= a.num) return;  // (a whole warp)
+    tlo_treelet(a, W[warp], i, lane, 32);
+}
+
 // NCCL, loaded on first use.  A process that already holds a libnccl.so.2 (torch brings its own) gets that one.
 struct Nccl {
     void *lib = nullptr;
@@ -1265,6 +1277,12 @@ struct CudaBackend {
         k_sah_small<<<count, kSahSmallWarps * 32, sizeof(SahSmallSmem), stream_>>>(a);
         RTB_CUDA_CHECK(cudaGetLastError());
     }
+    // treelet restructuring: the treelets of one depth (a.num roots)
+    void tlo_treelets(const TloArgs &a) {
+        if (a.num <= 0) return;
+        k_tlo_treelet<<<(a.num + kTloWarps - 1) / kTloWarps, kTloWarps * 32, 0, stream_>>>(a);
+        RTB_CUDA_CHECK(cudaGetLastError());
+    }
     // one level of the collapse over the work items counted in device memory (k.a.n_in_dev): a resident grid strides
     // over them; *zero is cleared for the level after the next, *levels counts the levels that had work
     void collapse_level(const CollapseK &k, int bound, int32_t *zero, int32_t *levels) {
@@ -1299,6 +1317,7 @@ struct CudaBackend {
 };
 
 static_assert(HasSahKernels<CudaBackend>::value, "the binned-SAH builder runs as k_sah_* kernels on the GPU");
+static_assert(HasTreeletKernels<CudaBackend>::value, "treelet restructuring runs as k_tlo_treelet on the GPU");
 
 }  // namespace rtb
 

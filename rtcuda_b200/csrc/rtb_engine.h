@@ -479,8 +479,13 @@ enum BuildCtr {
     kCtrSahBlocks = 13 /* 13,14,15: their blocks */, kCtrBounds = 16 /* 16..21 ordered floats, 22 = bad vertex */, kCtrTail = 24 /* 24: tail rounds, 25: root */,
     kCtrSahSmall = 26 /* small ranges */, kCtrCount = 32
 };
+// rtb_build_params.builder: the builder in the low byte, RTB_BUILDER_TREELET_PASSES(k) in bits 8..11
+inline int builder_kind(const rtb_build_params &bp) { return bp.builder & 0xff; }
+inline int treelet_passes(const rtb_build_params &bp) { return bp.builder >> 8 & 0xf; }
 inline void check_builder(const rtb_build_params &bp) {
-    if (bp.builder != RTB_BUILDER_PLOC && bp.builder != RTB_BUILDER_BINNED_SAH) throw Error(RTB_ERR_INVALID, "unknown BVH builder");
+    const int b = builder_kind(bp);
+    if ((bp.builder & ~0xfff) != 0 || (b != RTB_BUILDER_PLOC && b != RTB_BUILDER_BINNED_SAH) || treelet_passes(bp) > kTloMaxPasses)
+        throw Error(RTB_ERR_INVALID, "unknown BVH builder");
 }
 struct SetK {
     int32_t *p; int32_t v; int n;
@@ -601,6 +606,63 @@ SahOrder build_binned_sah(BE &be, Temps<BE> &tmp, int n, const F4 *prim_lo, cons
     o.order = order; o.first = first;
     return o;
 }
+// RTB_BUILDER_TREELET_PASSES: the treelets of one depth as a plain loop (the host emulation), or as the backend's
+// kernel; rtb_cuda.cu asserts that CudaBackend has one (k_tlo_treelet, one warp per treelet)
+template <class BE, class = void> struct HasTreeletKernels : std::false_type {};
+template <class BE>
+struct HasTreeletKernels<BE, std::void_t<decltype(std::declval<BE &>().tlo_treelets(std::declval<const TloArgs &>()))>> : std::true_type {};
+template <class BE>
+void tlo_treelets(BE &be, const TloArgs &a) {
+    if constexpr (HasTreeletKernels<BE>::value) {
+        be.tlo_treelets(a);
+    } else {
+        TloWork w;
+        for (int i = 0; i < a.num; ++i) tlo_treelet(a, w, i, 0, 1);
+    }
+}
+// inner nodes deepest first (order) and the host's copy of where each depth starts in it (as SahOrder::first)
+struct DepthOrder { const int32_t *order = nullptr; std::vector<int32_t> first; };
+// `passes` treelet passes over the binary tree (b2, count, root in *root_src) of n >= 2 primitives; with `plan`, the
+// depth order of the final tree for the collapse plan.  Per pass: depths, one sort, one read-back of the per-depth
+// table, then one launch per depth.
+template <class BE>
+DepthOrder run_treelet_passes(BE &be, Temps<BE> &tmp, int n, B2Node *b2, int32_t *count, const int32_t *root_src, int passes, bool plan) {
+    const int n_inner = n - 1;
+    TloArgs a{};
+    a.nodes = b2; a.count = count; a.root = root_src; a.n = n;
+    a.parent = tmp.template alloc<int32_t>((size_t)2 * n - 1);
+    a.depth = tmp.template alloc<int32_t>(n_inner);
+    uint64_t *keys = tmp.template alloc<uint64_t>(n_inner);
+    int32_t *order = tmp.template alloc<int32_t>(n_inner), *first = tmp.template alloc<int32_t>(kSahMaxDepth + 2);
+    a.order = order;
+    { TloParentK k; k.a = a; be.launch(n_inner, k); }
+    DepthOrder o;
+    o.first.resize(kSahMaxDepth + 2);
+    auto sort_by_depth = [&]() {
+        { TloDepthK k; k.a = a; be.launch(n_inner, k); }
+        { SahDepthKeyK k; k.depth = a.depth; k.keys = keys; k.vals = order; k.n_inner = n_inner; k.n = n; be.launch(n_inner, k); }
+        be.sort_pairs(keys, order, n_inner);
+        { SetK k; k.p = first; k.v = -1; k.n = kSahMaxDepth + 2; be.launch(k.n, k); }
+        { SahGroupK k; k.keys = keys; k.first = first; k.n_inner = n_inner; be.launch(n_inner, k); }
+        be.download(o.first.data(), first, o.first.size());
+        if (o.first[0] >= 0) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+    };
+    for (int p = 0; p < passes; ++p) {
+        sort_by_depth();
+        a.gamma = kTloGamma << p;
+        for (int k = 1; k <= kSahMaxDepth + 1; ++k) {  // deepest first
+            if (o.first[(size_t)k] < 0) continue;
+            int end = n_inner;
+            for (int j = k + 1; j <= kSahMaxDepth + 1; ++j) if (o.first[(size_t)j] >= 0) { end = o.first[(size_t)j]; break; }
+            a.first = o.first[(size_t)k]; a.num = end - a.first;
+            tlo_treelets(be, a);
+        }
+    }
+    if (plan) { sort_by_depth(); o.order = order; }
+    tmp.free(a.parent); tmp.free(a.depth); tmp.free(keys); tmp.free(first);
+    if (!plan) tmp.free(order);
+    return o;
+}
 constexpr int kMaxPlocLog = 1 << 16;
 template <class BE>
 BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriMeta *meta_in, const F4 *box_lo, const F4 *box_hi,
@@ -639,7 +701,22 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
     B2Node *b2 = tmp.template alloc<B2Node>(n_b2);
     int32_t *count = tmp.template alloc<int32_t>(n_b2);
     const bool want_plan = bp.collapse == RTB_COLLAPSE_SAH_OPTIMAL && n > max_leaf;
+    const int passes = n >= 2 ? treelet_passes(bp) : 0;
     float *plan_cost = nullptr; uint8_t *plan = nullptr;
+    // 4. collapse plan, one launch per depth, deepest first (a node's children are deeper): first[] as SahOrder::first
+    auto plan_by_depth = [&](const int32_t *order, const std::vector<int32_t> &first) {
+        if (first[0] >= 0) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+        plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
+        plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
+        for (int k = 1; k <= kSahMaxDepth + 1; ++k) {
+            if (first[(size_t)k] < 0) continue;
+            int end = n - 1;
+            for (int j = k + 1; j <= kSahMaxDepth + 1; ++j) if (first[(size_t)j] >= 0) { end = first[(size_t)j]; break; }
+            PlanK p; p.a.nodes = b2; p.a.count = count; p.a.cost = plan_cost; p.a.plan = plan;
+            p.a.first = first[(size_t)k]; p.a.n = end - first[(size_t)k]; p.a.max_leaf = max_leaf; p.a.order = order;
+            be.launch(p.a.n, p);
+        }
+    };
     const int32_t *root_src = ctr + kCtrTail + 1;
     int rounds = 0;
     bool tail = false;
@@ -658,7 +735,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
             if (h2[0]) be.download(htail.data(), be.ploc_tail_counts(), (size_t)h2[0]);
         }
     };
-    if (bp.builder == RTB_BUILDER_PLOC) {
+    if (builder_kind(bp) == RTB_BUILDER_PLOC) {
         const int radius = bp.ploc_radius > 0 ? bp.ploc_radius : 16;
         // 2. Morton codes + sort
         uint64_t *keys = tmp.template alloc<uint64_t>(n);
@@ -710,9 +787,10 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
         }
         if (!tail) root_src = ca;
         tmp.free(prim_lo); tmp.free(prim_hi); tmp.free(keys); tmp.free(sorted); tmp.free(nn);
-        // 4. collapse plan: bottom-up over the binary tree, one launch per PLOC round (a round's nodes only have older children)
-        if (want_plan) {
-            read_logs();
+        // 4. collapse plan: bottom-up over the binary tree, one launch per PLOC round (a round's nodes only have older
+        // children; after treelet passes they need not be, and the plan goes by depth below)
+        if (want_plan) read_logs();
+        if (want_plan && !passes) {
             plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
             plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
             int next_id = n;
@@ -729,25 +807,18 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
         }
     } else {
         // 2'-3'. binned SAH, top down; the root goes to ctr[kCtrTail + 1]
-        const SahOrder so = build_binned_sah(be, tmp, n, prim_lo, prim_hi, b2, count, ctr, want_plan);
-        const int32_t *order = so.order;
+        const SahOrder so = build_binned_sah(be, tmp, n, prim_lo, prim_hi, b2, count, ctr, want_plan && !passes);
         tmp.free(prim_lo); tmp.free(prim_hi);
-        // 4. collapse plan: one launch per depth, deepest first (a node's children are deeper)
-        if (want_plan) {
+        if (want_plan && !passes) {
             std::vector<int32_t> first(kSahMaxDepth + 2);
             be.download(first.data(), so.first, first.size());  // (the one read-back of the per-depth counts)
-            if (first[0] >= 0) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
-            plan_cost = tmp.template alloc<float>((size_t)n_b2 * 7);
-            plan = tmp.template alloc<uint8_t>((size_t)n_b2 * 8);
-            for (int k = 1; k <= kSahMaxDepth + 1; ++k) {
-                if (first[(size_t)k] < 0) continue;
-                int end = n - 1;
-                for (int j = k + 1; j <= kSahMaxDepth + 1; ++j) if (first[(size_t)j] >= 0) { end = first[(size_t)j]; break; }
-                PlanK p; p.a.nodes = b2; p.a.count = count; p.a.cost = plan_cost; p.a.plan = plan;
-                p.a.first = first[(size_t)k]; p.a.n = end - first[(size_t)k]; p.a.max_leaf = max_leaf; p.a.order = order;
-                be.launch(p.a.n, p);
-            }
+            plan_by_depth(so.order, first);
         }
+    }
+    // 3.5. treelet restructuring; the plan then goes by depth, whichever the builder
+    if (passes) {
+        const DepthOrder d = run_treelet_passes(be, tmp, n, b2, count, root_src, passes, want_plan);
+        if (want_plan) plan_by_depth(d.order, d.first);
     }
     // 5. collapse to the 8-wide compressed tree, level by level; the number of work items of a level stays on the
     // device (three rotating counters: read, written, cleared), the host reads it once per batch of levels
@@ -787,7 +858,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
     if (c[kCtrTri] != n) throw Error(RTB_ERR_INVALID, "internal: collapse lost triangles");
     out.nodes8 = be.template alloc<Q4>((size_t)out.num_nodes * kNodeWords);
     be.copy(out.nodes8, nodes_tmp, (size_t)out.num_nodes * kNodeWords);
-    if (bp.builder == RTB_BUILDER_PLOC && !want_plan) read_logs();
+    if (builder_kind(bp) == RTB_BUILDER_PLOC && !want_plan) read_logs();
     int iters = rounds > kMaxPlocLog ? rounds - kMaxPlocLog : 0;  // (rounds beyond the log are counted, not examined)
     for (size_t r = 0; r + 1 < hlog.size(); ++r) if (hlog[r] > hlog[r + 1]) ++iters;
     out.ploc_iterations = iters + (int)htail.size();

@@ -1,5 +1,6 @@
-"""A/B of the BVH builders: {PLOC, binned SAH} x {greedy, SAH-optimal collapse} on the C2 shape (S1, 1920x1080, 64 spp,
-depth 8) and the C3 shape (S2 grid 12, 3840x2160, 16 spp, depth 8).  One JSON line per variant:
+"""A/B of the BVH builders: {PLOC, binned SAH} x {greedy, SAH-optimal collapse} x --optimize (treelet passes,
+RTB_BUILDER_TREELET_PASSES) on the C2 shape (S1, 1920x1080, 64 spp, depth 8) and the C3 shape (S2 grid 12, 3840x2160,
+16 spp, depth 8).  One JSON line per variant:
 
   build_ms        median of 3 builds after one warm-up build (rtb_bvh_stats.build_ms, CUDA events)
   num_nodes, sah_cost
@@ -9,6 +10,7 @@ depth 8) and the C3 shape (S2 grid 12, 3840x2160, 16 spp, depth 8).  One JSON li
   ms_total        median of --steps renders, the variants of a workload alternated in one process
 
     python tools/builder_ab.py --steps 5 > profiles/r3/builder_ab.jsonl
+    python tools/builder_ab.py --steps 5 --optimize 0,3    # every variant without and with 3 treelet passes
 """
 import argparse
 import ctypes as C
@@ -55,8 +57,10 @@ def main():
     ap.add_argument("--workloads", default="c2,c3")
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--incoherent", type=int, default=500000)
+    ap.add_argument("--optimize", default="0", help="comma-separated treelet pass counts (0..8) to run every variant with")
     a = ap.parse_args()
     assert a.steps >= 5, "the render time is the median of at least 5 steps"
+    passes = [int(k) for k in a.optimize.split(",")]
     card, power = gpu_info()
     print(json.dumps({"card": card, "power_limit": power}), flush=True)
     L = capi.Lib()
@@ -70,10 +74,10 @@ def main():
         prim = L.primary_rays(cam, w, h)
         variants = []
         for bname, b in BUILDERS.items():
-            for cname, c in COLLAPSES.items():
+            for cname, c, k in [(cn, c, k) for cn, c in COLLAPSES.items() for k in passes]:
                 bp = capi.BuildParams()
                 L.lib.rtb_build_params_default(C.byref(bp))
-                bp.builder, bp.collapse = b, c
+                bp.builder, bp.collapse = b | capi.treelet_passes(k), c
                 ctx.scene(hs.desc, bp).close()  # warm-up build
                 times = []
                 for _ in range(3):
@@ -85,7 +89,7 @@ def main():
                 pn, pt = sc.trace_counts(prim)
                 inn, itr = sc.trace_counts(inc)
                 _, cs = sc.render(cam, capi.render_params(L, width=w, height=h, spp=1, max_bounces=depth, flags=capi.RTB_RENDER_COUNT_WORK))
-                rec = {"workload": wl, "builder": bname, "collapse": cname, "card": card, "power_limit": power,
+                rec = {"workload": wl, "builder": bname, "collapse": cname, "treelet_passes": k, "card": card, "power_limit": power,
                        "triangles": int(st.num_triangles), "build_ms": statistics.median(times), "build_ms_all": times,
                        "num_nodes": int(st.num_nodes), "collapse_levels": int(st.collapse_levels), "sah_cost": float(st.sah_cost),
                        "primary_nodes_per_ray": pn, "primary_tris_per_ray": pt, "incoherent_nodes_per_ray": inn, "incoherent_tris_per_ray": itr,

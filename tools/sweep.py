@@ -30,7 +30,7 @@ ap.add_argument("--device", type=int, default=0)
 ap.add_argument("--radius", type=int, default=0)
 ap.add_argument("--leaf", type=int, default=0)
 ap.add_argument("--collapse", type=int, default=-1)
-ap.add_argument("--builder", type=int, default=-1, help="rtb_build_params.builder (0 PLOC, 1 binned SAH)")
+ap.add_argument("--builder", type=int, default=-1, help="rtb_build_params.builder (0 PLOC, 1 binned SAH; + 256 * k for k treelet passes)")
 ap.add_argument("--count", action="store_true", help="also print nodes / triangles per ray (counting kernels)")
 ap.add_argument("--reps", type=int, default=2)
 ap.add_argument("--flags", type=int, default=0)
