@@ -290,6 +290,30 @@ RTB_API int rtb_scene_create_instanced(rtb_context *ctx, const rtb_instanced_sce
 RTB_API int rtb_scene_destroy(rtb_scene *scene);
 RTB_API int rtb_scene_stats(const rtb_scene *scene, rtb_bvh_stats *out);
 
+/* ---- updating a scene in place (animation) ---- */
+/* New vertex positions for every triangle (9 floats per triangle, caller order, as many triangles as at creation);
+ * topology, materials and lights unchanged.  The 8-wide tree keeps its topology and gets new boxes (refit), and the
+ * triangle records are derived from these vertices (also for a scene of rtb_scene_create_from_primitives, as the
+ * reference's host constructor derives them).  Instanced scenes: the geometry's object-space vertices; every mesh tree
+ * is refit and the tree over the instances is rebuilt with the current transforms.  Area lights follow their moved
+ * triangles.  A vertex that rtb_scene_create would reject (not finite, beyond 2^100), or a null pointer:
+ * RTB_ERR_INVALID and the scene is unchanged.  Afterwards rtb_bvh_stats.sah_cost and scene_bounds describe the refit
+ * tree; build_ms stays the time of the original build.
+ * A refit tree keeps the topology that was built for the original geometry: the further the geometry moves from that
+ * shape, the more nodes a ray visits and the slower traces and renders get (tools/refit_ab.py, DESIGN.md 4.9).
+ * Rebuild the scene (rtb_scene_create*) when that happens.  The render state of the scene (queues, accumulation
+ * buffer) is kept.  rtb_scene_refit_device reads the vertices from device memory on the scene's GPU, which must be
+ * ready when it is called (it runs on the context's stream); *ms (may be NULL) gets the GPU time of the update. */
+RTB_API int rtb_scene_refit(rtb_scene *scene, const float *h_vertices);
+RTB_API int rtb_scene_refit_device(rtb_scene *scene, const float *d_vertices, float *ms);
+/* Instanced scenes only: new instance records, as many as at creation; instance i keeps its mesh (so the flattened hit
+ * ids keep their meaning), its transform and material may change.  The instance boxes and the tree over the instances
+ * are rebuilt; the mesh trees are untouched.  The checks of rtb_scene_create_instanced apply (transform finite and
+ * invertible, material in range, a mesh with emitters keeps its single identity placement, stack depth); on failure
+ * RTB_ERR_INVALID and the scene is unchanged.  Afterwards rtb_bvh_stats.num_nodes, num_top_nodes, collapse_levels,
+ * sah_cost and scene_bounds describe the new tree. */
+RTB_API int rtb_scene_set_instances(rtb_scene *scene, const rtb_instance *h_instances, int32_t num_instances);
+
 /* ---- ray queries (replace Bvh::traverse closest-hit bvh.cuh:251-303 with
  *      kernel ch render.cuh:297-328, and any-hit bvh.cuh:306-357 with kernel
  *      ah render.cuh:278-294) ---- */

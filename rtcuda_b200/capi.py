@@ -108,6 +108,7 @@ SYMBOLS = [
     "rtb_multi_scene_create_instanced", "rtb_multi_scene_replicate", "rtb_multi_scene_destroy", "rtb_multi_render", "rtb_render_multi",
     "rtb_scene_attach_lights", "rtb_accum_create", "rtb_accum_destroy", "rtb_accum_add_samples", "rtb_accum_samples",
     "rtb_accum_resolve", "rtb_accum_save", "rtb_accum_load", "rtb_comm_unique_id", "rtb_comm_create", "rtb_comm_destroy", "rtb_comm_allreduce_f32", "rtb_comm_allreduce_i64",
+    "rtb_scene_refit", "rtb_scene_refit_device", "rtb_scene_set_instances",
 ]
 RTB_COMM_ID_BYTES = 128
 RTB_KAT_TRI_INTERSECT, RTB_KAT_OFFSET_ORIGIN, RTB_KAT_RAND4, RTB_KAT_SAMPLE_F, RTB_KAT_SLAB, RTB_KAT_SAMPLE_LI = 1, 2, 3, 4, 5, 6
@@ -341,6 +342,25 @@ class Scene:
         self.L.check(self.L.lib.rtb_trace_closest_counts(self.h, rays.ctypes.data_as(C.c_void_p),
                                                          C.c_int64(len(rays)), C.byref(a), C.byref(b)))
         return a.value, b.value
+
+    def refit(self, verts):
+        """new vertex positions (float32 [num_triangles, 9], caller order; object space for an instanced scene): the tree
+        keeps its topology and gets new boxes (rtb_scene_refit)"""
+        verts = np.ascontiguousarray(verts, dtype=np.float32)
+        if verts.size != 9 * self.stats().num_triangles:
+            raise RtbError(f"refit: {verts.size} floats for {self.stats().num_triangles} triangles (9 per triangle)")
+        self.L.check(self.L.lib.rtb_scene_refit(self.h, verts.ctypes.data_as(C.c_void_p)))
+
+    def refit_device(self, d_vertices_ptr):
+        """rtb_scene_refit_device from 9 floats per triangle in device memory (ready on the device); returns its GPU ms"""
+        ms = C.c_float()
+        self.L.check(self.L.lib.rtb_scene_refit_device(self.h, C.c_void_p(d_vertices_ptr), C.byref(ms)))
+        return ms.value
+
+    def set_instances(self, instances):
+        """new transforms / materials for the instances of an instanced scene (a ctypes array of Instance, same count,
+        same meshes): rtb_scene_set_instances"""
+        self.L.check(self.L.lib.rtb_scene_set_instances(self.h, C.cast(instances, C.c_void_p), len(instances)))
 
     def render_aovs(self, cam, width, height):
         """primary-hit feature buffers: (albedo[h,w,3], normal[h,w,3], depth[h,w], prim[h,w])"""

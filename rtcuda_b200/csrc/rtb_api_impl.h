@@ -108,6 +108,31 @@ int rtb_scene_create_instanced(rtb_context *ctx, const rtb_instanced_scene_desc 
         *out = new rtb_scene{ctx, impl};
     });
 }
+int rtb_scene_refit(rtb_scene *s, const float *h_vertices) {
+    if (!s) return rtb::set_error(RTB_ERR_INVALID, "rtb_scene_refit: null scene");
+    return rtb::guarded([&] {
+        s->ctx->be.make_current();
+        s->ctx->be.use_stream(0);
+        rtb::refit_scene(s->ctx->be, *s->impl, h_vertices, nullptr);
+    });
+}
+int rtb_scene_refit_device(rtb_scene *s, const float *d_vertices, float *ms) {
+    if (!s) return rtb::set_error(RTB_ERR_INVALID, "rtb_scene_refit_device: null scene");
+    return rtb::guarded([&] {
+        s->ctx->be.make_current();
+        s->ctx->be.use_stream(0);
+        const float e = rtb::refit_scene(s->ctx->be, *s->impl, nullptr, d_vertices);
+        if (ms) *ms = e;
+    });
+}
+int rtb_scene_set_instances(rtb_scene *s, const rtb_instance *h_instances, int32_t num_instances) {
+    if (!s) return rtb::set_error(RTB_ERR_INVALID, "rtb_scene_set_instances: null scene");
+    return rtb::guarded([&] {
+        s->ctx->be.make_current();
+        s->ctx->be.use_stream(0);
+        rtb::set_instances(s->ctx->be, *s->impl, h_instances, num_instances);
+    });
+}
 int rtb_scene_destroy(rtb_scene *s) {
     return rtb::guarded([&] {
         if (!s) return;

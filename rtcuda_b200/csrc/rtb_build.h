@@ -80,6 +80,7 @@ constexpr float kMaxCoord = 1.2676506e30f;
 // bounds of one triangle record, the vertex check and the scene bounds; t is triangle i's record (already stored)
 RTB_HD void prim_setup_bounds(const PrimSetupArgs &a, int i, const Tri48 &t);
 RTB_HD void prim_setup_box(const PrimSetupArgs &a, int i, const Tri48 &t, V3 &lo, V3 &hi);
+RTB_HD bool tri_box(const Tri48 &t, V3 &lo, V3 &hi);
 RTB_HD void prim_setup_body(const PrimSetupArgs &a, int i) {
     if (i >= a.n) return;
     Tri48 t;
@@ -116,6 +117,13 @@ RTB_HD void prim_setup_bounds(const PrimSetupArgs &a, int i, const Tri48 &t) {
 #endif
 }
 RTB_HD void prim_setup_box(const PrimSetupArgs &a, int i, const Tri48 &t, V3 &lo, V3 &hi) {
+    if (tri_box(t, lo, hi)) *a.bad = 1;
+    F4 l; l.x = lo.x; l.y = lo.y; l.z = lo.z; l.w = 0.f;
+    F4 h; h.x = hi.x; h.y = hi.y; h.z = hi.z; h.w = 0.f;
+    a.prim_lo[i] = l; a.prim_hi[i] = h;
+}
+// box of one triangle record (the builder's and the refit's); true when a vertex is not finite or beyond kMaxCoord
+RTB_HD bool tri_box(const Tri48 &t, V3 &lo, V3 &hi) {
     // Triangle::bounding_box, triangle.cuh:23-37 (p1 = p0 - e1, p2 = p0 + e2)
     V3 p0 = tri_p0(t), p1 = vsub(p0, tri_e1(t)), p2 = vadd(p0, tri_e2(t));
     lo = v3(fminf(p0.x, fminf(p1.x, p2.x)), fminf(p0.y, fminf(p1.y, p2.y)), fminf(p0.z, fminf(p1.z, p2.z)));
@@ -125,10 +133,7 @@ RTB_HD void prim_setup_box(const PrimSetupArgs &a, int i, const Tri48 &t, V3 &lo
                               fmaxf(fmaxf(fabsf(p1.y), fabsf(p1.z)), fmaxf(fabsf(p2.x), fmaxf(fabsf(p2.y), fabsf(p2.z)))));
     const bool nan = p0.x != p0.x || p0.y != p0.y || p0.z != p0.z || p1.x != p1.x || p1.y != p1.y || p1.z != p1.z || p2.x != p2.x ||
                      p2.y != p2.y || p2.z != p2.z;
-    if (nan || !(worst <= kMaxCoord)) *a.bad = 1;
-    F4 l; l.x = lo.x; l.y = lo.y; l.z = lo.z; l.w = 0.f;
-    F4 h; h.x = hi.x; h.y = hi.y; h.z = hi.z; h.w = 0.f;
-    a.prim_lo[i] = l; a.prim_hi[i] = h;
+    return nan || !(worst <= kMaxCoord);
 }
 
 // ------------------------------------------------------------ 2. morton
@@ -731,6 +736,8 @@ struct CollapseArgs {
     float *sah;                // accumulated SAH cost (unnormalised)
     int32_t max_leaf;          // 1..3
     int32_t *gather;           // [n] leaf order: binary subtree whose triangles start at this slot, or -1 (gather_body)
+    int32_t *level_nodes;      // null, or where this level records its number of work items = 8-wide nodes of its depth
+                               // (the depth schedule of the refit: a level's nodes are one contiguous range of ids)
 };
 // triangles of the leaf children, in leaf order: slot d holds the binary subtree whose (<= 3) triangles go to d, d+1, ..
 // (left to right) or -1; one thread per slot, after the collapse
@@ -758,7 +765,9 @@ RTB_HD void gather_body(const CollapseArgs &a, int n, int d) {
 }
 
 RTB_HD void collapse_body(const CollapseArgs &a, int tid) {
-    if (tid >= (a.n_in_dev ? *a.n_in_dev : a.n_in)) return;
+    const int n_in = a.n_in_dev ? *a.n_in_dev : a.n_in;
+    if (tid >= n_in) return;
+    if (tid == 0 && a.level_nodes) *a.level_nodes = n_in;
     const WorkItem item = a.work_in[tid];
     const B2Node self = a.nodes[item.b2];
     int ch[8];
@@ -891,6 +900,97 @@ RTB_HD void collapse_body(const CollapseArgs &a, int tid) {
 #undef RTB_PACK4
     Q4 *dst = a.nodes8 + (size_t)item.wide * kNodeWords;
     dst[0] = w0; dst[1] = w1; dst[2] = w2; dst[3] = w3; dst[4] = w4;
+}
+
+// ------------------------------------------------------------ 6. refit (rtb_scene_refit)
+// New vertices, same topology.  The record pass turns caller-order vertices into the records at leaf_of_prim[i], with the
+// vertex check of prim_setup.  The refit pass then goes one depth at a time, deepest first, and recomputes each node
+// from its own words: a leaf child's box is the union of its triangles' boxes (tri_box), an inner child's box is the
+// exact box the deeper level left in `box`, and the node's origin, exponents and quantised planes are rewritten with the
+// functions of collapse_body (child_base, tri_base, meta and imask stay).  The collapse's frame is its binary node's
+// box, which is the union of the triangle boxes below it: with the original vertices the refit writes the same words.
+struct RefitTrisArgs {
+    const float *vertices;         // 9 per triangle, caller order
+    const int32_t *leaf_of_prim;   // caller index -> leaf order
+    F4 *tris;                      // [n] leaf order, 3 words per triangle (whole 16-byte stores: the writes scatter)
+    int32_t *bad;                  // raised when a vertex is not finite or beyond kMaxCoord
+    int32_t n;
+};
+RTB_HD void refit_tris_body(const RefitTrisArgs &a, int i) {
+    if (i >= a.n) return;
+    const float *v = a.vertices + 9 * (size_t)i;
+    const Tri48 t = tri_from_vertices(v3(v[0], v[1], v[2]), v3(v[3], v[4], v[5]), v3(v[6], v[7], v[8]));
+    V3 lo, hi;
+    if (tri_box(t, lo, hi)) *a.bad = 1;
+    F4 *d = a.tris + 3 * (size_t)a.leaf_of_prim[i];
+    F4 w;
+    w.x = t.p0x; w.y = t.p0y; w.z = t.p0z; w.w = t.e1x; d[0] = w;
+    w.x = t.e1y; w.y = t.e1z; w.z = t.e2x; w.w = t.e2y; d[1] = w;
+    w.x = t.e2z; w.y = t.nx; w.z = t.ny; w.w = t.nz; d[2] = w;
+}
+struct RefitArgs {
+    Q4 *nodes8;
+    const F4 *tris;           // leaf order, 3 words per triangle
+    float *box;               // [nodes][6]: exact box (lo xyz, hi xyz) of every node refit so far
+    const int32_t *order;     // null: this launch refits nodes first .. first + num - 1; else order[first .. first + num)
+    int32_t first, num;
+    float *sah;               // accumulated 8-wide SAH cost (unnormalised), as collapse_body sums it
+};
+// refits one node; returns its term of the SAH cost
+RTB_HD float refit_body(const RefitArgs &a, int tid) {
+    const int id = a.order ? a.order[a.first + tid] : a.first + tid;
+    Q4 *nd = a.nodes8 + (size_t)id * kNodeWords;
+    const Q4 w0 = nd[0], w1 = nd[1];
+    const uint32_t imask = w0.w >> 24;
+    V3 clo[8], chi[8];
+    int cnt[8];  // triangles of a leaf child, 0: inner child or empty slot
+    V3 lo = v3(FLT_MAX), hi = v3(-FLT_MAX);
+#pragma unroll
+    for (int s = 0; s < 8; ++s) {
+        const uint32_t m = ((s < 4 ? w1.z : w1.w) >> (8 * (s & 3))) & 0xffu;
+        cnt[s] = 0;
+        clo[s] = v3(FLT_MAX); chi[s] = v3(-FLT_MAX);
+        if (imask >> s & 1u) {
+            const float *b = a.box + 6 * (size_t)(w1.x + (uint32_t)popc(imask & ((1u << s) - 1u)));
+            clo[s] = v3(b[0], b[1], b[2]); chi[s] = v3(b[3], b[4], b[5]);
+        } else if (m) {
+            cnt[s] = popc(m >> 5);
+            for (int t = 0; t < cnt[s]; ++t) {
+                V3 l, h;
+                tri_box(load_tri(a.tris, (int)(w1.y + (m & 31u)) + t), l, h);
+                clo[s] = v3(fminf(clo[s].x, l.x), fminf(clo[s].y, l.y), fminf(clo[s].z, l.z));
+                chi[s] = v3(fmaxf(chi[s].x, h.x), fmaxf(chi[s].y, h.y), fmaxf(chi[s].z, h.z));
+            }
+        } else {
+            continue;
+        }
+        lo = v3(fminf(lo.x, clo[s].x), fminf(lo.y, clo[s].y), fminf(lo.z, clo[s].z));
+        hi = v3(fmaxf(hi.x, chi[s].x), fmaxf(hi.y, chi[s].y), fmaxf(hi.z, chi[s].z));
+    }
+    const uint32_t ex = quant_exponent(fsub(hi.x, lo.x)), ey = quant_exponent(fsub(hi.y, lo.y)), ez = quant_exponent(fsub(hi.z, lo.z));
+    uint32_t qlx[8], qly[8], qlz[8], qhx[8], qhy[8], qhz[8];
+    float sah = fmul(half_area(fsub(hi.x, lo.x), fsub(hi.y, lo.y), fsub(hi.z, lo.z)), kSahNodeCost);
+#pragma unroll
+    for (int s = 0; s < 8; ++s) {
+        const bool used = cnt[s] > 0 || (imask >> s & 1u);
+        qlx[s] = used ? quant_lo(clo[s].x, lo.x, ex) : 255u; qhx[s] = used ? quant_hi(chi[s].x, lo.x, ex) : 0u;
+        qly[s] = used ? quant_lo(clo[s].y, lo.y, ey) : 255u; qhy[s] = used ? quant_hi(chi[s].y, lo.y, ey) : 0u;
+        qlz[s] = used ? quant_lo(clo[s].z, lo.z, ez) : 255u; qhz[s] = used ? quant_hi(chi[s].z, lo.z, ez) : 0u;
+        if (cnt[s] > 0)
+            sah = ffma(half_area(fsub(chi[s].x, clo[s].x), fsub(chi[s].y, clo[s].y), fsub(chi[s].z, clo[s].z)), fmul(kSahTriCost, (float)cnt[s]), sah);
+    }
+    float *b = a.box + 6 * (size_t)id;
+    b[0] = lo.x; b[1] = lo.y; b[2] = lo.z; b[3] = hi.x; b[4] = hi.y; b[5] = hi.z;
+    Q4 o0, w2, w3, w4;
+    o0.x = f2u(lo.x); o0.y = f2u(lo.y); o0.z = f2u(lo.z);
+    o0.w = ex | (ey << 8) | (ez << 16) | (imask << 24);
+#define RTB_PACK4(q, o) ((q)[o] | ((q)[o + 1] << 8) | ((q)[o + 2] << 16) | ((q)[o + 3] << 24))
+    w2.x = RTB_PACK4(qlx, 0); w2.y = RTB_PACK4(qlx, 4); w2.z = RTB_PACK4(qly, 0); w2.w = RTB_PACK4(qly, 4);
+    w3.x = RTB_PACK4(qlz, 0); w3.y = RTB_PACK4(qlz, 4); w3.z = RTB_PACK4(qhx, 0); w3.w = RTB_PACK4(qhx, 4);
+    w4.x = RTB_PACK4(qhy, 0); w4.y = RTB_PACK4(qhy, 4); w4.z = RTB_PACK4(qhz, 0); w4.w = RTB_PACK4(qhz, 4);
+#undef RTB_PACK4
+    nd[0] = o0; nd[2] = w2; nd[3] = w3; nd[4] = w4;
+    return sah;
 }
 
 // ------------------------------------------------------------ two-level scenes

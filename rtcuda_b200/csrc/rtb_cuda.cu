@@ -855,6 +855,17 @@ __global__ void __launch_bounds__(kTloWarps * 32) k_tlo_treelet(TloArgs a) {
     tlo_treelet(a, W[warp], i, lane, 32);
 }
 
+// ---- refit (rtb_scene_refit, rtb_build.h 6) ----
+// The nodes of one depth, one thread each.  Every lane of a block exists (the grid is rounded up, out-of-range lanes
+// contribute 0), so the SAH terms are summed over the full warp mask and one lane per warp adds them to the total.
+__global__ void __launch_bounds__(kBlock) k_refit_level(RefitArgs a) {
+    const int i = blockIdx.x * kBlock + threadIdx.x;
+    float v = i < a.num ? refit_body(a, i) : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0 && v != 0.f) atomicAdd(a.sah, v);
+}
+
 // NCCL, loaded on first use.  A process that already holds a libnccl.so.2 (torch brings its own) gets that one.
 struct Nccl {
     void *lib = nullptr;
@@ -1292,6 +1303,13 @@ struct CudaBackend {
         RTB_CUDA_CHECK(cudaGetLastError());
     }
 
+    // refit: the nodes of one depth (a.num of them)
+    void refit_level(const RefitArgs &a) {
+        if (a.num <= 0) return;
+        k_refit_level<<<(a.num + kBlock - 1) / kBlock, kBlock, 0, stream_>>>(a);
+        RTB_CUDA_CHECK(cudaGetLastError());
+    }
+
     using Time = cudaEvent_t;
     Time now() {
         cudaEvent_t e;
@@ -1318,6 +1336,7 @@ struct CudaBackend {
 
 static_assert(HasSahKernels<CudaBackend>::value, "the binned-SAH builder runs as k_sah_* kernels on the GPU");
 static_assert(HasTreeletKernels<CudaBackend>::value, "treelet restructuring runs as k_tlo_treelet on the GPU");
+static_assert(HasRefitKernels<CudaBackend>::value, "the refit runs as k_refit_level on the GPU");
 
 }  // namespace rtb
 

@@ -350,6 +350,17 @@ struct SceneT {
     // in caller order, and the base of the caller's triangle array (area lights name their triangle by pointer)
     const void **deferred_light_ptr = nullptr; const char *ref_tri_base = nullptr;
     rtb_bvh_stats stats{};
+    // in-place updates (refit_scene, set_instances).  The collapse levels of every tree: one tree for a flat scene, one
+    // per mesh for an instanced scene, whose mesh trees start at tree_first[m] after the top tree's nodes
+    rtb_build_params bp{};
+    std::vector<std::vector<int32_t>> tree_levels;
+    std::vector<int32_t> tree_first;
+    // instanced scenes: the description's meshes and instances, which meshes hold emitters, the material types
+    std::vector<int64_t> mesh_first;
+    std::vector<rtb_instance> instances;
+    std::vector<uint8_t> mesh_emissive;
+    std::vector<int32_t> material_type;
+    int mesh_levels = 0;
     // render state kept between calls (the reference re-allocates ~293 MB per
     // render() and never frees it, render.cuh:374-391)
     WaveState W[kMaxPipelines]{};
@@ -446,6 +457,7 @@ struct BuiltTree {
     Q4 *nodes8 = nullptr;
     int32_t num_nodes = 0;
     int levels = 0, ploc_iterations = 0;
+    std::vector<int32_t> level_nodes;  // nodes of each collapse level (depth): level L is ids [sum of the levels before, + count)
     float sah_cost = 0.f;
     float bounds[6] = {0, 0, 0, 0, 0, 0};  // xmin xmax ymin ymax zmin zmax
 };
@@ -477,7 +489,8 @@ enum BuildCtr {
     kCtrB2 = 0, kCtrWide = 1, kCtrTri = 2, kCtrNcl = 4, kCtrLevels = 5, kCtrLvl0 = 6 /* 6,7,8: work items of a level, rotating */,
     kCtrSah = 9 /* float */, kCtrSahTasks = 10 /* 10,11,12: large ranges of a level, rotating */,
     kCtrSahBlocks = 13 /* 13,14,15: their blocks */, kCtrBounds = 16 /* 16..21 ordered floats, 22 = bad vertex */, kCtrTail = 24 /* 24: tail rounds, 25: root */,
-    kCtrSahSmall = 26 /* small ranges */, kCtrCount = 32
+    kCtrSahSmall = 26 /* small ranges */,
+    kCtrLevelNodes = 32 /* 32 .. 32 + kStackSize - 1: 8-wide nodes of each collapse level */, kCtrCount = 32 + kStackSize
 };
 // rtb_build_params.builder: the builder in the low byte, RTB_BUILDER_TREELET_PASSES(k) in bits 8..11
 inline int builder_kind(const rtb_build_params &bp) { return bp.builder & 0xff; }
@@ -841,6 +854,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
             k.a.leaf_of_prim = leaf_of_prim; k.a.node_counter = ctr + kCtrWide; k.a.tri_counter = ctr + kCtrTri;
             k.a.work_in = wa; k.a.n_in = 0; k.a.n_in_dev = ctr + kCtrLvl0 + level % 3; k.a.work_out = wb;
             k.a.n_out = ctr + kCtrLvl0 + (level + 1) % 3; k.a.sah = sah; k.a.max_leaf = max_leaf; k.a.gather = gather;
+            k.a.level_nodes = level < kStackSize ? ctr + kCtrLevelNodes + level : nullptr;  // (deeper trees are rejected)
             ga = k.a;
             be.collapse_level(k, max_nodes, ctr + kCtrLvl0 + (level + 2) % 3, ctr + kCtrLevels);
             WorkItem *t = wa; wa = wb; wb = t;
@@ -855,6 +869,7 @@ BuiltTree build_tree(BE &be, int n, const float *d_vertices, Tri48 *tri_in, TriM
     be.download(c, ctr, kCtrCount);
     out.num_nodes = c[kCtrWide];
     out.levels = c[kCtrLevels];
+    out.level_nodes.assign(c + kCtrLevelNodes, c + kCtrLevelNodes + (out.levels < kStackSize ? out.levels : kStackSize));
     if (c[kCtrTri] != n) throw Error(RTB_ERR_INVALID, "internal: collapse lost triangles");
     out.nodes8 = be.template alloc<Q4>((size_t)out.num_nodes * kNodeWords);
     be.copy(out.nodes8, nodes_tmp, (size_t)out.num_nodes * kNodeWords);
@@ -908,6 +923,9 @@ void build_bvh(BE &be, SceneT<BE> &sc, const float *d_vertices, Tri48 *tri_in, T
     sc.nodes8 = bt.nodes8;
     sc.num_nodes = bt.num_nodes;
     if (bt.levels >= kStackSize) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+    sc.bp = bp;
+    sc.tree_levels.assign(1, bt.level_nodes);
+    sc.tree_first.assign(1, 0);
     if (sc.num_lights > 0) {
         LightFixK k; k.lights = sc.lights; k.light_tri = d_light_tri; k.leaf_of_prim = sc.leaf_of_prim; k.n = sc.num_lights;
         be.launch(sc.num_lights, k);
@@ -1166,6 +1184,123 @@ inline bool is_identity3x4(const float *m) {
     for (int k = 0; k < 12; ++k) if (m[k] != id[k]) return false;
     return true;
 }
+// mesh, material and transform of one instance; its world -> object matrix into inv
+inline void check_instance(const rtb_instance &in, int num_meshes, int num_materials, double *inv) {
+    if (in.mesh < 0 || in.mesh >= num_meshes) throw Error(RTB_ERR_INVALID, "instance: mesh out of range");
+    if (in.material < -1 || in.material >= num_materials) throw Error(RTB_ERR_INVALID, "instance: material out of range");
+    for (int k = 0; k < 12; ++k) if (!std::isfinite(in.xform[k])) throw Error(RTB_ERR_INVALID, "instance: transform not finite");
+    if (!invert3x4(in.xform, inv)) throw Error(RTB_ERR_INVALID, "instance: transform not invertible");
+}
+// The tree over the instances and everything that depends on it, for the instances in sc.instances (checked, with their
+// world -> object matrices in `inverse`): the instances' world boxes from the triangles `tris` (leaf order), the top
+// tree, the stack-depth check, one node array (the top tree, then the mesh trees of `mesh_nodes`, whose indices are
+// rebased to a top tree of `mesh_base` nodes, re-rebased to the new one) and the instance records.  Everything is built
+// before anything of the scene is replaced; the scene's old arrays are freed after.  Scene creation and
+// rtb_scene_set_instances both come here.
+template <class BE>
+void install_top(BE &be, SceneT<BE> &sc, const std::vector<double> &inverse, const Q4 *mesh_nodes, int32_t mesh_base,
+                 int32_t num_mesh_nodes, const F4 *tris) {
+    const int ni = (int)sc.instances.size();
+    Temps<BE> tmp(be);
+    // the instances' world boxes, from the transformed vertices of their meshes, padded by more than the rounding of
+    // the ray transform can move a hit point (1e-5 of the coordinates' magnitude)
+    std::vector<F4> blo((size_t)ni), bhi((size_t)ni);
+    {
+        std::vector<float> xf(12 * (size_t)ni);
+        std::vector<int32_t> ifirst((size_t)ni), icount((size_t)ni), binit(6 * (size_t)ni), bout(6 * (size_t)ni);
+        int largest = 1;
+        for (int i = 0; i < ni; ++i) {
+            const rtb_instance &in = sc.instances[(size_t)i];
+            memcpy(&xf[12 * (size_t)i], in.xform, sizeof(float) * 12);
+            ifirst[(size_t)i] = (int32_t)sc.mesh_first[(size_t)in.mesh];
+            icount[(size_t)i] = (int32_t)(sc.mesh_first[(size_t)in.mesh + 1] - sc.mesh_first[(size_t)in.mesh]);
+            if (icount[(size_t)i] > largest) largest = icount[(size_t)i];
+            for (int k = 0; k < 3; ++k) { binit[6 * (size_t)i + k] = float_to_ordered(FLT_MAX); binit[6 * (size_t)i + 3 + k] = float_to_ordered(-FLT_MAX); }
+        }
+        InstBoundsK k;
+        k.a.runs = (largest + kInstBoundsRun - 1) / kInstBoundsRun;
+        if ((long long)k.a.runs * ni > 0x7fffffffll) throw Error(RTB_ERR_INVALID, "too many instances x triangles for the bounds pass");
+        float *d_xf = tmp.template alloc<float>(xf.size());
+        int32_t *d_first = tmp.template alloc<int32_t>(ni), *d_count = tmp.template alloc<int32_t>(ni), *d_b = tmp.template alloc<int32_t>(6 * (size_t)ni);
+        be.upload(d_xf, xf.data(), xf.size()); be.upload(d_first, ifirst.data(), (size_t)ni); be.upload(d_count, icount.data(), (size_t)ni);
+        be.upload(d_b, binit.data(), binit.size());
+        k.a.tris = (const Tri48 *)tris; k.a.xforms = d_xf; k.a.first = d_first; k.a.count = d_count; k.a.bounds = d_b; k.a.num_inst = ni;
+        be.launch(k.a.runs * ni, k);
+        be.download(bout.data(), d_b, bout.size());
+        tmp.free(d_xf); tmp.free(d_first); tmp.free(d_count); tmp.free(d_b);
+        for (int i = 0; i < ni; ++i) {
+            float lo[3], hi[3];
+            double mag = 0.0;
+            for (int k2 = 0; k2 < 3; ++k2) {
+                lo[k2] = ordered_to_float(bout[6 * (size_t)i + k2]); hi[k2] = ordered_to_float(bout[6 * (size_t)i + 3 + k2]);
+                mag = fmax(mag, fmax(fabs((double)lo[k2]), fabs((double)hi[k2])));
+            }
+            const double pad = 1e-5 * mag + 1e-30;
+            F4 l, h;
+            l.x = (float)(lo[0] - pad); l.y = (float)(lo[1] - pad); l.z = (float)(lo[2] - pad); l.w = 0.f;
+            h.x = (float)(hi[0] + pad); h.y = (float)(hi[1] + pad); h.z = (float)(hi[2] + pad); h.w = 0.f;
+            if (!(fabsf(l.x) <= FLT_MAX && fabsf(l.y) <= FLT_MAX && fabsf(l.z) <= FLT_MAX && fabsf(h.x) <= FLT_MAX && fabsf(h.y) <= FLT_MAX && fabsf(h.z) <= FLT_MAX))
+                throw Error(RTB_ERR_INVALID, "instance: world box not finite");
+            blo[(size_t)i] = l; bhi[(size_t)i] = h;
+        }
+    }
+    F4 *d_blo = tmp.template alloc<F4>(ni), *d_bhi = tmp.template alloc<F4>(ni);
+    be.upload(d_blo, blo.data(), (size_t)ni); be.upload(d_bhi, bhi.data(), (size_t)ni);
+    DeviceBuf<BE, int32_t> top_inst(be, (size_t)ni);
+    int32_t *top_leaf_of = tmp.template alloc<int32_t>(ni);
+    // every instance gets a child box of its own in the top tree (leaf lists of one entry)
+    // (the SAH-optimal collapse: its tie-breaking caveat concerns triangles, and it halves the top tree — S2: 57 -> 27
+    // nodes, 3.55 -> 3.38 nodes per primary ray; leaf lists of 2 or 3 instances were measured worse)
+    rtb_build_params tbp = sc.bp;
+    tbp.collapse = RTB_COLLAPSE_SAH_OPTIMAL;
+    const BuiltTree top = build_tree(be, ni, nullptr, nullptr, nullptr, d_blo, d_bhi, tbp, 1, nullptr, nullptr, top_inst.p, top_leaf_of);
+    DeviceBuf<BE, Q4> top_nodes(be, 0);
+    top_nodes.p = top.nodes8;
+    tmp.free(d_blo); tmp.free(d_bhi); tmp.free(top_leaf_of);
+    // stack: a node group per level of both trees, plus the rest of a leaf list per level of the top tree
+    if (2 * top.levels + sc.mesh_levels >= kStackSize) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
+    // one node array: the top tree, then the meshes' trees rebased by the change of the top tree's size
+    const int32_t num_nodes = top.num_nodes + num_mesh_nodes;
+    DeviceBuf<BE, Q4> nodes(be, (size_t)num_nodes * kNodeWords);
+    be.copy(nodes.p, top.nodes8, (size_t)top.num_nodes * kNodeWords);
+    {
+        RebaseK k; k.src = mesh_nodes; k.dst = nodes.p + (size_t)top.num_nodes * kNodeWords;
+        k.node_off = (uint32_t)(top.num_nodes - mesh_base); k.tri_off = 0u; k.n = num_mesh_nodes;  // (a smaller top tree: wraps, as intended)
+        be.launch(k.n, k);
+    }
+    // instance records
+    std::vector<F4> rec((size_t)ni * kInstWords);
+    int64_t flat_first = 0;
+    for (int i = 0; i < ni; ++i) {
+        const rtb_instance &in = sc.instances[(size_t)i];
+        const double *inv = &inverse[12 * (size_t)i];
+        F4 *r = rec.data() + (size_t)i * kInstWords;
+        for (int k = 0; k < 3; ++k) {
+            r[k].x = (float)inv[4 * k]; r[k].y = (float)inv[4 * k + 1]; r[k].z = (float)inv[4 * k + 2]; r[k].w = (float)inv[4 * k + 3];
+            r[3 + k].x = in.xform[4 * k]; r[3 + k].y = in.xform[4 * k + 1]; r[3 + k].z = in.xform[4 * k + 2]; r[3 + k].w = in.xform[4 * k + 3];
+        }
+        const int mat = in.material >= 0 ? (in.material | (sc.material_type[(size_t)in.material] << 24)) : -1;
+        r[6].x = i2f(top.num_nodes + sc.tree_first[(size_t)in.mesh]); r[6].y = i2f(mat); r[6].z = i2f((int)flat_first);
+        r[6].w = i2f((int)sc.mesh_first[(size_t)in.mesh]);
+        r[7].x = r[7].y = r[7].z = r[7].w = 0.f;
+        flat_first += sc.mesh_first[(size_t)in.mesh + 1] - sc.mesh_first[(size_t)in.mesh];
+    }
+    DeviceBuf<BE, F4> inst(be, (size_t)ni * kInstWords);
+    be.upload(inst.p, rec.data(), rec.size());
+    be.sync();
+    // nothing below throws: the new arrays replace the old ones
+    be.free(sc.nodes8); be.free(sc.inst); be.free(sc.top_inst);
+    sc.nodes8 = nodes.release(); sc.inst = inst.release(); sc.top_inst = top_inst.release();
+    sc.num_nodes = num_nodes;
+    sc.num_inst = ni;
+    sc.stats.num_nodes = num_nodes;
+    sc.stats.node_bytes = (int64_t)num_nodes * 80;
+    sc.stats.sah_cost = top.sah_cost;
+    sc.stats.ploc_iterations = top.ploc_iterations;
+    sc.stats.collapse_levels = top.levels + sc.mesh_levels;
+    for (int k = 0; k < 6; ++k) sc.stats.scene_bounds[k] = top.bounds[k];
+    sc.stats.num_top_nodes = top.num_nodes;
+}
 template <class BE>
 SceneT<BE> *scene_from_instanced(BE &be, const rtb_instanced_scene_desc &D, const rtb_build_params &bp) {
     const rtb_scene_desc &d = D.geometry;
@@ -1186,10 +1321,7 @@ SceneT<BE> *scene_from_instanced(BE &be, const rtb_instanced_scene_desc &D, cons
     std::vector<double> inverse(12 * (size_t)ni);  // world -> object, checked before any device work
     for (int i = 0; i < ni; ++i) {
         const rtb_instance &in = D.instances[i];
-        if (in.mesh < 0 || in.mesh >= nm) throw Error(RTB_ERR_INVALID, "instance: mesh out of range");
-        if (in.material < -1 || in.material >= d.num_materials) throw Error(RTB_ERR_INVALID, "instance: material out of range");
-        for (int k = 0; k < 12; ++k) if (!std::isfinite(in.xform[k])) throw Error(RTB_ERR_INVALID, "instance: transform not finite");
-        if (!invert3x4(in.xform, &inverse[12 * (size_t)i])) throw Error(RTB_ERR_INVALID, "instance: transform not invertible");
+        check_instance(in, nm, d.num_materials, &inverse[12 * (size_t)i]);
         uses[(size_t)in.mesh]++;
         if (!is_identity3x4(in.xform)) ident[(size_t)in.mesh] = 0;
         flat_first[(size_t)i + 1] = flat_first[(size_t)i] + (D.mesh_first[in.mesh + 1] - D.mesh_first[in.mesh]);
@@ -1227,7 +1359,6 @@ SceneT<BE> *scene_from_instanced(BE &be, const rtb_instanced_scene_desc &D, cons
     const int max_leaf = bp.max_leaf_tris >= 1 && bp.max_leaf_tris <= 3 ? bp.max_leaf_tris : 3;
     SceneT<BE> *sc = new SceneT<BE>();
     std::vector<BuiltTree> trees((size_t)nm);
-    BuiltTree top;
     try {
         sc->be = &be;
         sc->n = n;
@@ -1265,121 +1396,184 @@ SceneT<BE> *scene_from_instanced(BE &be, const rtb_instanced_scene_desc &D, cons
             if (trees[(size_t)m].levels > mesh_levels) mesh_levels = trees[(size_t)m].levels;
         }
         tmp.free(d_vertices); tmp.free(tri_in); tmp.free(meta_in);
-        // the instances' world boxes, from the transformed vertices of their meshes, padded by more than the rounding of
-        // the ray transform can move a hit point (1e-5 of the coordinates' magnitude)
-        std::vector<F4> blo((size_t)ni), bhi((size_t)ni);
+        // what updates of the scene need (refit_scene, set_instances)
+        sc->bp = bp;
+        sc->mesh_first.assign(D.mesh_first, D.mesh_first + nm + 1);
+        sc->instances.assign(D.instances, D.instances + ni);
+        sc->mesh_emissive.assign((size_t)nm, 0);
+        for (int i = 0; i < n; ++i) if (meta[(size_t)i].light >= 0) sc->mesh_emissive[(size_t)mesh_of[(size_t)i]] = 1;
+        for (int i = 0; i < d.num_lights; ++i)
+            if (d.lights[i].type == RTB_AREA_LIGHT) sc->mesh_emissive[(size_t)mesh_of[(size_t)d.lights[i].triangle]] = 1;
+        sc->material_type.resize((size_t)d.num_materials);
+        for (int i = 0; i < d.num_materials; ++i) sc->material_type[(size_t)i] = d.materials[i].type;
+        sc->mesh_levels = mesh_levels;
+        // the meshes' trees in one array, rebased as if the top tree had no nodes (install_top moves them behind it)
+        Q4 *mesh_nodes_d = tmp.template alloc<Q4>((size_t)mesh_nodes * kNodeWords);
+        sc->tree_levels.resize((size_t)nm);
+        sc->tree_first.resize((size_t)nm);
         {
-            std::vector<float> xf(12 * (size_t)ni);
-            std::vector<int32_t> ifirst((size_t)ni), icount((size_t)ni), binit(6 * (size_t)ni), bout(6 * (size_t)ni);
-            int largest = 1;
-            for (int i = 0; i < ni; ++i) {
-                const rtb_instance &in = D.instances[i];
-                memcpy(&xf[12 * (size_t)i], in.xform, sizeof(float) * 12);
-                ifirst[(size_t)i] = (int32_t)D.mesh_first[in.mesh];
-                icount[(size_t)i] = (int32_t)(D.mesh_first[in.mesh + 1] - D.mesh_first[in.mesh]);
-                if (icount[(size_t)i] > largest) largest = icount[(size_t)i];
-                for (int k = 0; k < 3; ++k) { binit[6 * (size_t)i + k] = float_to_ordered(FLT_MAX); binit[6 * (size_t)i + 3 + k] = float_to_ordered(-FLT_MAX); }
+            int off = 0;
+            for (int m = 0; m < nm; ++m) {
+                RebaseK k; k.src = trees[(size_t)m].nodes8; k.dst = mesh_nodes_d + (size_t)off * kNodeWords;
+                k.node_off = (uint32_t)off; k.tri_off = (uint32_t)D.mesh_first[m]; k.n = trees[(size_t)m].num_nodes;
+                be.launch(k.n, k);
+                sc->tree_first[(size_t)m] = off;
+                sc->tree_levels[(size_t)m] = trees[(size_t)m].level_nodes;
+                off += trees[(size_t)m].num_nodes;
             }
-            InstBoundsK k;
-            k.a.runs = (largest + kInstBoundsRun - 1) / kInstBoundsRun;
-            if ((long long)k.a.runs * ni > 0x7fffffffll) throw Error(RTB_ERR_INVALID, "too many instances x triangles for the bounds pass");
-            float *d_xf = tmp.template alloc<float>(xf.size());
-            int32_t *d_first = tmp.template alloc<int32_t>(ni), *d_count = tmp.template alloc<int32_t>(ni), *d_b = tmp.template alloc<int32_t>(6 * (size_t)ni);
-            be.upload(d_xf, xf.data(), xf.size()); be.upload(d_first, ifirst.data(), (size_t)ni); be.upload(d_count, icount.data(), (size_t)ni);
-            be.upload(d_b, binit.data(), binit.size());
-            k.a.tris = (const Tri48 *)sc->tris; k.a.xforms = d_xf; k.a.first = d_first; k.a.count = d_count; k.a.bounds = d_b; k.a.num_inst = ni;
-            be.launch(k.a.runs * ni, k);
-            be.download(bout.data(), d_b, bout.size());
-            tmp.free(d_xf); tmp.free(d_first); tmp.free(d_count); tmp.free(d_b);
-            for (int i = 0; i < ni; ++i) {
-                float lo[3], hi[3];
-                double mag = 0.0;
-                for (int k2 = 0; k2 < 3; ++k2) {
-                    lo[k2] = ordered_to_float(bout[6 * (size_t)i + k2]); hi[k2] = ordered_to_float(bout[6 * (size_t)i + 3 + k2]);
-                    mag = fmax(mag, fmax(fabs((double)lo[k2]), fabs((double)hi[k2])));
-                }
-                const double pad = 1e-5 * mag + 1e-30;
-                F4 l, h;
-                l.x = (float)(lo[0] - pad); l.y = (float)(lo[1] - pad); l.z = (float)(lo[2] - pad); l.w = 0.f;
-                h.x = (float)(hi[0] + pad); h.y = (float)(hi[1] + pad); h.z = (float)(hi[2] + pad); h.w = 0.f;
-                if (!(fabsf(l.x) <= FLT_MAX && fabsf(l.y) <= FLT_MAX && fabsf(l.z) <= FLT_MAX && fabsf(h.x) <= FLT_MAX && fabsf(h.y) <= FLT_MAX && fabsf(h.z) <= FLT_MAX))
-                    throw Error(RTB_ERR_INVALID, "instance: world box not finite");
-                blo[(size_t)i] = l; bhi[(size_t)i] = h;
-            }
-        }
-        F4 *d_blo = tmp.template alloc<F4>(ni), *d_bhi = tmp.template alloc<F4>(ni);
-        be.upload(d_blo, blo.data(), (size_t)ni); be.upload(d_bhi, bhi.data(), (size_t)ni);
-        sc->top_inst = be.template alloc<int32_t>(ni);
-        int32_t *top_leaf_of = tmp.template alloc<int32_t>(ni);
-        // every instance gets a child box of its own in the top tree (leaf lists of one entry)
-        // (the SAH-optimal collapse: its tie-breaking caveat concerns triangles, and it halves the top tree — S2: 57 -> 27
-        // nodes, 3.55 -> 3.38 nodes per primary ray; leaf lists of 2 or 3 instances were measured worse)
-        rtb_build_params tbp = bp;
-        tbp.collapse = RTB_COLLAPSE_SAH_OPTIMAL;
-        top = build_tree(be, ni, nullptr, nullptr, nullptr, d_blo, d_bhi, tbp, 1, nullptr, nullptr, sc->top_inst, top_leaf_of);
-        tmp.free(d_blo); tmp.free(d_bhi); tmp.free(top_leaf_of);
-        // stack: a node group per level of both trees, plus the rest of a leaf list per level of the top tree
-        if (2 * top.levels + mesh_levels >= kStackSize) throw Error(RTB_ERR_INVALID, "BVH too deep for the traversal stack");
-        // one node array: the top tree, then the meshes' trees rebased
-        sc->num_nodes = top.num_nodes + mesh_nodes;
-        sc->nodes8 = be.template alloc<Q4>((size_t)sc->num_nodes * kNodeWords);
-        be.copy(sc->nodes8, top.nodes8, (size_t)top.num_nodes * kNodeWords);
-        std::vector<int> root_of((size_t)nm);
-        int off = top.num_nodes;
-        for (int m = 0; m < nm; ++m) {
-            RebaseK k; k.src = trees[(size_t)m].nodes8; k.dst = sc->nodes8 + (size_t)off * kNodeWords;
-            k.node_off = (uint32_t)off; k.tri_off = (uint32_t)D.mesh_first[m]; k.n = trees[(size_t)m].num_nodes;
-            be.launch(k.n, k);
-            root_of[(size_t)m] = off;
-            off += trees[(size_t)m].num_nodes;
         }
         be.sync();
         for (int m = 0; m < nm; ++m) { be.free(trees[(size_t)m].nodes8); trees[(size_t)m].nodes8 = nullptr; }
-        be.free(top.nodes8); top.nodes8 = nullptr;
-        // instance records
-        std::vector<F4> rec((size_t)ni * kInstWords);
-        for (int i = 0; i < ni; ++i) {
-            const rtb_instance &in = D.instances[i];
-            const double *inv = &inverse[12 * (size_t)i];
-            F4 *r = rec.data() + (size_t)i * kInstWords;
-            for (int k = 0; k < 3; ++k) {
-                r[k].x = (float)inv[4 * k]; r[k].y = (float)inv[4 * k + 1]; r[k].z = (float)inv[4 * k + 2]; r[k].w = (float)inv[4 * k + 3];
-                r[3 + k].x = in.xform[4 * k]; r[3 + k].y = in.xform[4 * k + 1]; r[3 + k].z = in.xform[4 * k + 2]; r[3 + k].w = in.xform[4 * k + 3];
-            }
-            const int mat = in.material >= 0 ? (in.material | (d.materials[in.material].type << 24)) : -1;
-            r[6].x = i2f(root_of[(size_t)in.mesh]); r[6].y = i2f(mat); r[6].z = i2f((int)flat_first[(size_t)i]); r[6].w = i2f((int)D.mesh_first[in.mesh]);
-            r[7].x = r[7].y = r[7].z = r[7].w = 0.f;
-        }
-        sc->inst = be.template alloc<F4>((size_t)ni * kInstWords);
-        be.upload(sc->inst, rec.data(), rec.size());
-        sc->num_inst = ni;
+        sc->stats = rtb_bvh_stats{};
+        install_top(be, *sc, inverse, mesh_nodes_d, 0, mesh_nodes, sc->tris);
+        tmp.free(mesh_nodes_d);
         if (sc->num_lights > 0) {
             LightFixK k; k.lights = sc->lights; k.light_tri = d_light_tri; k.leaf_of_prim = sc->leaf_of_prim; k.n = sc->num_lights;
             be.launch(sc->num_lights, k);
         }
         be.sync();
         tmp.free(d_light_tri);
-        sc->stats = rtb_bvh_stats{};
         sc->stats.num_triangles = n;
         sc->stats.num_bvh2_nodes = 2 * (int64_t)n - nm + 2 * (int64_t)ni - 1;
-        sc->stats.num_nodes = sc->num_nodes;
-        sc->stats.node_bytes = (int64_t)sc->num_nodes * 80;
         sc->stats.triangle_bytes = (int64_t)n * 48;
-        sc->stats.sah_cost = top.sah_cost;
-        sc->stats.ploc_iterations = top.ploc_iterations;
-        sc->stats.collapse_levels = top.levels + mesh_levels;
-        for (int k = 0; k < 6; ++k) sc->stats.scene_bounds[k] = top.bounds[k];
         sc->stats.num_instances = ni;
         sc->stats.num_flat_triangles = sc->n_flat;
-        sc->stats.num_top_nodes = top.num_nodes;
         sc->stats.build_ms = be.elapsed_ms(t0, be.now());
     } catch (...) {
         for (auto &t : trees) be.free(t.nodes8);
-        be.free(top.nodes8);
         delete sc;
         throw;
     }
     return sc;
+}
+
+// ---- in-place updates (rtb_scene_refit, rtb_scene_set_instances) ----
+struct RefitTrisK { RefitTrisArgs a; RTB_HD void operator()(int i) const { refit_tris_body(a, i); } };
+// The nodes of one depth: the backend's kernel (rtb_cuda.cu asserts that CudaBackend has one: k_refit_level, whose warps
+// reduce the SAH terms over a full mask before one atomic), or a plain loop (the host emulation).
+template <class BE, class = void> struct HasRefitKernels : std::false_type {};
+template <class BE>
+struct HasRefitKernels<BE, std::void_t<decltype(std::declval<BE &>().refit_level(std::declval<const RefitArgs &>()))>> : std::true_type {};
+template <class BE>
+void refit_level(BE &be, const RefitArgs &a) {
+    if constexpr (HasRefitKernels<BE>::value) be.refit_level(a);
+    else for (int i = 0; i < a.num; ++i) atomic_add_f(a.sah, refit_body(a, i));
+}
+// New vertex positions for every triangle (9 floats each, caller order; host or device memory), same topology.  Returns
+// the GPU time of the update.  Every temporary is allocated first, and the scene is only touched once the vertices
+// have passed the builder's check.  The records go to a new array that replaces the scene's (rather than a check-only
+// pass over the vertices and an in-place write): an instanced scene needs the new records for the instance boxes before
+// its top tree is rebuilt, and that rebuild may still fail (a world box beyond float, the stack depth), which must
+// leave the scene as it was; reading the vertices once also keeps the large flat scenes at one pass over them.  The
+// spare records cost the size of the triangle array while the call runs (S2: 480 MB of a B200's 180 GB).
+template <class BE>
+float refit_scene(BE &be, SceneT<BE> &sc, const float *h_vertices, const float *d_vertices) {
+    const int n = (int)sc.n;
+    if (n > 0 && !h_vertices && !d_vertices) throw Error(RTB_ERR_INVALID, "rtb_scene_refit: null vertices");
+    if (n == 0) return 0.f;  // (the empty root has nothing to refit)
+    const bool inst = sc.inst != nullptr;
+    const int top_nodes = inst ? (int)sc.stats.num_top_nodes : 0;
+    // depth schedule: the nodes of each depth, deepest first.  A flat scene's are one range per level; an instanced
+    // scene's are the union of its mesh trees' ranges, as a list of ids
+    int depths = 0;
+    for (const auto &lv : sc.tree_levels) depths = (int)lv.size() > depths ? (int)lv.size() : depths;
+    std::vector<int32_t> ids, dfirst((size_t)depths + 1, 0);
+    {
+        int64_t total = 0;
+        for (size_t t = 0; t < sc.tree_levels.size(); ++t) for (int32_t c : sc.tree_levels[t]) total += c;
+        if (total != (int64_t)sc.num_nodes - top_nodes) throw Error(RTB_ERR_INVALID, "internal: refit depth schedule does not cover the tree");
+        // per depth (ascending) and tree: the range's first id
+        std::vector<std::vector<int32_t>> first(sc.tree_levels.size());
+        for (size_t t = 0; t < sc.tree_levels.size(); ++t) {
+            int32_t f = top_nodes + sc.tree_first[t];
+            for (int32_t c : sc.tree_levels[t]) { first[t].push_back(f); f += c; }
+        }
+        if (inst) {
+            for (int d = depths - 1, k = 0; d >= 0; --d, ++k) {
+                dfirst[(size_t)k] = (int32_t)ids.size();
+                for (size_t t = 0; t < sc.tree_levels.size(); ++t)
+                    if (d < (int)sc.tree_levels[t].size())
+                        for (int32_t j = 0; j < sc.tree_levels[t][(size_t)d]; ++j) ids.push_back(first[t][(size_t)d] + j);
+            }
+            dfirst[(size_t)depths] = (int32_t)ids.size();
+        } else {
+            for (int d = depths - 1, k = 0; d >= 0; --d, ++k) dfirst[(size_t)k] = first[0][(size_t)d];
+        }
+    }
+    Temps<BE> tmp(be);
+    float *vup = h_vertices ? tmp.template alloc<float>(9 * (size_t)n) : nullptr;
+    Tri48 *tris = tmp.template alloc<Tri48>(n);
+    int32_t *ctr = tmp.template alloc<int32_t>(2);  // bad vertex, SAH sum (float)
+    float *box = tmp.template alloc<float>(6 * (size_t)sc.num_nodes);
+    Q4 *nodes = inst ? tmp.template alloc<Q4>((size_t)sc.num_nodes * kNodeWords) : sc.nodes8;  // (instanced: a copy, see above)
+    int32_t *d_ids = inst ? tmp.template alloc<int32_t>(ids.size()) : nullptr;
+    std::vector<double> inverse(12 * sc.instances.size());  // (instanced: the scene's instances, checked when they were set)
+    for (size_t i = 0; i < sc.instances.size(); ++i) invert3x4(sc.instances[i].xform, &inverse[12 * i]);
+    if (h_vertices) be.upload(vup, h_vertices, 9 * (size_t)n);
+    if (inst) be.upload(d_ids, ids.data(), ids.size());
+    auto t0 = be.now();
+    try {
+        be.zero(ctr, 2);
+        {
+            RefitTrisK k; k.a.vertices = h_vertices ? vup : d_vertices; k.a.leaf_of_prim = sc.leaf_of_prim; k.a.tris = (F4 *)tris; k.a.bad = ctr; k.a.n = n;
+            be.launch(n, k);
+        }
+        int32_t bad = 0;
+        be.download(&bad, ctr, 1);
+        if (bad) throw Error(RTB_ERR_INVALID, "rtb_scene_refit: a triangle vertex is not finite or beyond 2^100; the scene is unchanged");
+        if (inst) be.copy(nodes, sc.nodes8, (size_t)sc.num_nodes * kNodeWords);
+        for (int k = 0; k < depths; ++k) {
+            RefitArgs a; a.nodes8 = nodes; a.tris = (const F4 *)tris; a.box = box; a.sah = (float *)(ctr + 1);
+            a.order = d_ids;
+            if (inst) { a.first = dfirst[(size_t)k]; a.num = dfirst[(size_t)k + 1] - dfirst[(size_t)k]; }
+            else { a.first = dfirst[(size_t)k]; a.num = sc.tree_levels[0][(size_t)(depths - 1 - k)]; }
+            refit_level(be, a);
+        }
+        if (inst) {
+            install_top(be, sc, inverse, nodes + (size_t)top_nodes * kNodeWords, top_nodes, sc.num_nodes - top_nodes, (const F4 *)tris);
+        } else {
+            float c[7];
+            be.download(c, box, 6);
+            be.download(c + 6, (const float *)(ctr + 1), 1);
+            const float root_area = half_area(c[3] - c[0], c[4] - c[1], c[5] - c[2]);
+            sc.stats.sah_cost = root_area > 0.f ? c[6] / root_area : 0.f;
+            for (int k = 0; k < 3; ++k) { sc.stats.scene_bounds[2 * k] = c[k]; sc.stats.scene_bounds[2 * k + 1] = c[3 + k]; }
+        }
+    } catch (...) {
+        be.release(t0);
+        throw;
+    }
+    // the new records replace the old ones (flat scenes: the nodes were refit in place; instanced: install_top)
+    for (auto &h : tmp.held) if (h == (void *)tris) h = (void *)sc.tris;  // (the old records are freed with the temporaries)
+    sc.tris = (F4 *)tris;
+    return be.elapsed_ms(t0, be.now());
+}
+// New instance records for an instanced scene: same count, every instance keeps its mesh (so the flattened hit ids keep
+// their meaning), transforms and materials may change.  The mesh trees stay; the instance boxes, the top tree and the
+// records are rebuilt (install_top).
+template <class BE>
+void set_instances(BE &be, SceneT<BE> &sc, const rtb_instance *h_instances, int32_t num_instances) {
+    if (!sc.inst) throw Error(RTB_ERR_INVALID, "rtb_scene_set_instances: not an instanced scene");
+    if (!h_instances) throw Error(RTB_ERR_INVALID, "rtb_scene_set_instances: null instances");
+    if (num_instances != (int32_t)sc.instances.size()) throw Error(RTB_ERR_INVALID, "rtb_scene_set_instances: the instance count differs from the scene's");
+    const int ni = num_instances, nm = (int)sc.mesh_first.size() - 1;
+    std::vector<double> inverse(12 * (size_t)ni);
+    for (int i = 0; i < ni; ++i) {
+        const rtb_instance &in = h_instances[i];
+        if (in.mesh != sc.instances[(size_t)i].mesh) throw Error(RTB_ERR_INVALID, "rtb_scene_set_instances: instance: mesh changed");
+        check_instance(in, nm, sc.num_materials, &inverse[12 * (size_t)i]);
+        if (sc.mesh_emissive[(size_t)in.mesh] && !is_identity3x4(in.xform))
+            throw Error(RTB_ERR_INVALID, "rtb_scene_set_instances: an emissive triangle must belong to a mesh instanced exactly once with the identity transform");
+    }
+    const std::vector<rtb_instance> old = sc.instances;
+    sc.instances.assign(h_instances, h_instances + ni);
+    const int top_nodes = (int)sc.stats.num_top_nodes;
+    try {
+        install_top(be, sc, inverse, sc.nodes8 + (size_t)top_nodes * kNodeWords, top_nodes, sc.num_nodes - top_nodes, sc.tris);
+    } catch (...) {
+        sc.instances = old;
+        throw;
+    }
 }
 
 // ---- wavefront loop ----
